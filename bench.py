@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step returned, DIR/*.npy
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d row C2): OS2015 academic multiscale example, 8x8
 subdomains, 6144 fine DG dofs each, local basis size 20 (n_red = 1280), Q = 2 affine terms; online batch of
@@ -91,7 +92,16 @@ def parse_args():
     ap.add_argument('--synthetic3d', default=None, metavar='HX,HY,HZ',
                     help='seeded synthetic operators with 3D structure (config C4 shape): --subdomains per direction, '
                          'HX x HY x HZ cells of 4 dofs per subdomain (16,16,12 -> n_i = 12288); offline measurements only')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='after the timed steps, write what the last online step returned (u, eta, info, eta_max, and '
+                         'the parameters mu they belong to) as DIR/<name>.npy in float64; at most 64 MB, a fixed seeded '
+                         'sample of the parameters when all of them would not fit (rank 0 only)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and (a.impl != 'b200' or a.offline_only):
+        ap.error('--dump-outputs writes the outputs of the online step of --impl b200; it cannot be combined with '
+                 '--impl reference or --offline-only')
     if a.config == 'c3':
         a.problem, a.subdomains, a.n_mu, a.c5 = 'spe10', 16, 2048, False
     elif a.config == 'c4':
@@ -389,7 +399,7 @@ def measure_offline(a, torch, planner, d, bases, fp64_peak, flush_l2, t_reduce_f
     for _ in range(max(3, a.warmup)):
         planner.run()
     times_all, times_proj = [], []
-    for _ in range(max(3, a.steps)):
+    for _ in range(a.steps):
         flush_l2()
         e0, e1, e2 = (torch.cuda.Event(enable_timing=True) for _ in range(3))
         e0.record()
@@ -471,7 +481,7 @@ def measure_sharded_offline(a, torch, dist, d, bases, flush_l2, barrier, ms_unsh
     for _ in range(3):
         ps.run(); ps.exchange()
     t_run, t_all = [], []
-    for _ in range(max(3, a.steps)):
+    for _ in range(a.steps):
         flush_l2()
         barrier()
         e0, e1, e2 = (torch.cuda.Event(enable_timing=True) for _ in range(3))
@@ -485,7 +495,7 @@ def measure_sharded_offline(a, torch, dist, d, bases, flush_l2, barrier, ms_unsh
     # the same exchange through NCCL (one in-place all-gather), timed beside the peer-memory path
     from pylrbms_b200.distributed import exchange_kind, exchange_regions
     t_nccl = []
-    for it in range(3 + max(3, a.steps)):
+    for it in range(3 + a.steps):
         flush_l2()
         barrier()
         e0, e1 = (torch.cuda.Event(enable_timing=True) for _ in range(2))
@@ -599,6 +609,28 @@ def sparse_solve_gate(rd, mus, n_check=2):
             'residual_rel': worst_r}
 
 
+DUMP_BYTES = 48 << 20          # --dump-outputs stays below 64 MB in all
+
+
+def dump_outputs(out_dir, mus, u, eta, info, mx, am):
+    """Write what one online step returned -- reduced solutions ``u`` (n_mu x n_red), ``eta``, the factorisation flags
+    ``info`` and ``eta_max`` = [max, argmax] -- with the parameters ``mu`` they belong to, as float64 ``<name>.npy`` files.
+    When every parameter's row does not fit ``DUMP_BYTES``, the rows of a fixed, seeded sample of the parameters are
+    written (their positions in the batch are ``index``), so that two runs with the same arguments compare row for row."""
+    import torch
+    n_mu, n_red = u.shape
+    rows = max(1, DUMP_BYTES // (8 * (n_red + 4)))
+    idx = np.arange(n_mu) if rows >= n_mu else np.sort(np.random.default_rng(0).choice(n_mu, rows, replace=False))
+    sel = torch.from_numpy(idx).to(u.device)
+    arrays = {'index': idx.astype(np.float64), 'mu': np.asarray(mus, dtype=np.float64)[idx],
+              'u': u.index_select(0, sel).cpu().numpy(), 'eta': eta.index_select(0, sel).cpu().numpy(),
+              'info': info.index_select(0, sel).cpu().numpy().astype(np.float64),
+              'eta_max': np.array([float(mx.item()), float(am.item())])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), x)
+
+
 def run_b200(a):
     import torch
     import torch.distributed as dist
@@ -660,7 +692,7 @@ def run_b200(a):
             for _ in range(3):
                 p3.run()
             t3 = []
-            for _ in range(max(3, a.steps)):
+            for _ in range(a.steps):
                 flush_l2()
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record(); p3.run(); e1.record(); e1.synchronize()
@@ -695,7 +727,7 @@ def run_b200(a):
         mx, am = rd.eta_max_device(eta)
         if world > 1:
             dist.all_reduce(mx, op=dist.ReduceOp.MAX)
-        return ev_mid, mx
+        return ev_mid, mx, am
 
     for _ in range(max(3, a.warmup)):
         step()
@@ -709,12 +741,14 @@ def run_b200(a):
         flush_l2()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        ev_mid, mx = step()
+        ev_mid, mx, am = step()
         e1.record()
         e1.synchronize()
         t_step.append(e0.elapsed_time(e1)); t_solve.append(e0.elapsed_time(ev_mid))
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, mus, u, eta, info, mx, am)
     if int(info.abs().max().item()) != 0:
         raise SystemExit('bench.py: a reduced system was flagged as not positive definite')
     total_ms = torch.tensor([float(np.sum(t_step))], dtype=torch.float64, device='cuda')
@@ -724,7 +758,7 @@ def run_b200(a):
     value = world * n_mu * a.steps / total_s
 
     # ---- end to end through the public API: host parameters -> host results, copies inside the timed region
-    e2e_steps = max(2, min(a.steps, 5))
+    e2e_steps = a.steps
     if a.eta_only:
         eta_host = torch.empty(n_mu, dtype=torch.float64).pin_memory()
 
@@ -777,7 +811,7 @@ def run_b200(a):
         c5_call()
         barrier()
         t0 = time.perf_counter()
-        reps5 = 2
+        reps5 = a.steps
         for _ in range(reps5):
             gmax, garg = c5_call()
         barrier()

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- runs the REFERENCE'S OWN source files for the hot path on seeded inputs.
 
 ``estimators.py``, ``reductor.py`` and ``online_enrichment.py`` of the reference are loaded *unmodified* from
-``/root/reference/python/dune/pylrbms`` (never copied) and executed on top of stand-ins for their third-party
+``$LRBMS_REFERENCE_DIR`` (a pylrbms checkout's ``python/dune/pylrbms``, never copied) and executed on top of stand-ins for their third-party
 dependencies, none of which can be installed here:
 
 * **pyMOR** (the fork ``git+https://zivgitlab.uni-muenster.de/srave_01/pymor.git@master``, pymor-0.5, branch-pinned only):
@@ -19,7 +19,7 @@ eta, the indicators), the reductor (``reductor.py:32-73``: Oswald / flux-reconst
 the reduced ``fr_red`` / ``oi_red`` operators), Doerfler marking and the enrichment loop (``online_enrichment.py:9-93``).
 What it does not pin: pyMOR's projection / unblock / Gram-Schmidt algorithms (restated, see above) and anything DUNE
 assembles.  ``tests/golden/make_reference_golden.py`` writes the outputs as fixtures; ``tests/test_oracle_golden.py``
-checks the oracle's own restatement of those files against them without needing ``/root/reference``.
+checks the oracle's own restatement of those files against them without needing the reference.
 """
 from __future__ import annotations
 
@@ -33,7 +33,8 @@ import types
 
 import numpy as np
 
-REFERENCE_DIR = '/root/reference/python/dune/pylrbms'
+# the ``python/dune/pylrbms`` directory of a pylrbms checkout; the reference is not part of this repository
+REFERENCE_DIR = os.environ.get('LRBMS_REFERENCE_DIR', '')
 
 
 class _Logger(logging.Logger):
@@ -139,7 +140,8 @@ def load_reference(reference_dir=REFERENCE_DIR):
     """The reference's three modules, executed from where they lie.  Returns a namespace with ``estimators``, ``reductor``,
     ``online_enrichment``."""
     if not os.path.isdir(reference_dir):
-        raise FileNotFoundError(reference_dir + ' is not available (the reference only exists in the build container)')
+        raise FileNotFoundError('reference sources not found at {!r}: set LRBMS_REFERENCE_DIR to the python/dune/pylrbms '
+                                'directory of a pylrbms checkout'.format(reference_dir))
     install_dependency_stand_ins()
     out = types.SimpleNamespace()
     for name in ('estimators', 'reductor', 'online_enrichment'):

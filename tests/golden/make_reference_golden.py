@@ -1,8 +1,8 @@
 """Generate ``reference_run__*.npz``: outputs of the REFERENCE'S OWN ``estimators.py`` / ``reductor.py`` /
-``online_enrichment.py`` (loaded unmodified from ``/root/reference``, see ``oracle/reference_run.py``) on the seeded
+``online_enrichment.py`` (loaded unmodified from ``$LRBMS_REFERENCE_DIR``, see ``oracle/reference_run.py``) on the seeded
 inputs of ``make_golden.py``.
 
-    python tests/golden/make_reference_golden.py          # only where /root/reference exists (the build container)
+    LRBMS_REFERENCE_DIR=<pylrbms checkout>/python/dune/pylrbms python tests/golden/make_reference_golden.py
 
 The reference's third-party layers (pyMOR fork, dune-gdt, mpi4py) are not installable; they are replaced by the NumPy
 stand-ins named in ``oracle/reference_run.py``.  So these vectors pin the arithmetic that lives in the reference's own

@@ -4,6 +4,8 @@ symbolic phase produces a schedule that reproduces a dense Cholesky when replaye
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -32,19 +34,31 @@ def test_binding_covers_header(built_library):
     assert lib.lrbms_version() == 100
 
 
+_NO_DEVICE_CHECK = '''
+import ctypes as C
+import sys
+sys.path.insert(0, sys.argv[1])
+from pylrbms_b200 import _lib
+lib = _lib.load_library()
+h = C.c_void_p()
+rc = lib.lrbms_create(0, C.byref(h))
+assert rc == -3 and not h.value, rc                  # LRBMS_ERR_NO_DEVICE
+assert b'no CPU fallback' in lib.lrbms_last_error(None)
+try:
+    _lib.Handle.get()
+except _lib.LrbmsError:
+    pass
+else:
+    raise AssertionError('Handle.get() succeeded without a device')
+'''
+
+
 def test_no_cpu_fallback(built_library):
-    """Without a CUDA device a handle cannot be created and the package raises instead of falling back."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip('a GPU is present')
-    from pylrbms_b200 import _lib
-    lib = _lib.load_library()
-    h = C.c_void_p()
-    rc = lib.lrbms_create(0, C.byref(h))
-    assert rc == -3 and not h.value                      # LRBMS_ERR_NO_DEVICE
-    assert b'no CPU fallback' in lib.lrbms_last_error(None)
-    with pytest.raises(_lib.LrbmsError):
-        _lib.Handle.get()
+    """Without a CUDA device a handle cannot be created and the package raises instead of falling back.  Checked in a child
+    process that sees no device (CUDA_VISIBLE_DEVICES empty), so that it also runs where a GPU is present."""
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES='')
+    r = subprocess.run([sys.executable, '-c', _NO_DEVICE_CHECK, ROOT], env=env, capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def _grid_blocks(sx, sy):

@@ -96,6 +96,33 @@ def test_bench_flop_model_matches_survey():
     assert abs(fl['solve'] - (0.46e6 + 41.5e6 + 0.92e6)) < 0.1e6
 
 
+@pytest.mark.parametrize('n_mu,n_red', [(7, 5), (10000, 1280)])
+def test_bench_dump_outputs(tmp_path, n_mu, n_red):
+    """``bench.py --dump-outputs``: float64 .npy files under 64 MB in all; above the budget the same seeded parameter sample
+    every time, rows consistent with the batch they were taken from."""
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    mus = np.linspace(0.1, 1.0, n_mu)
+    u = torch.arange(n_mu * n_red, dtype=torch.float64).reshape(n_mu, n_red)
+    eta = torch.from_numpy(mus ** 2)
+    info = torch.zeros(n_mu, dtype=torch.int32)
+    mx, am = eta.max().reshape(1), eta.argmax().reshape(1)
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), mus, u, eta, info, mx, am)
+    names = sorted(p.name for p in (tmp_path / 'a').iterdir())
+    assert names == ['eta.npy', 'eta_max.npy', 'index.npy', 'info.npy', 'mu.npy', 'u.npy']
+    assert sum((tmp_path / 'a' / n).stat().st_size for n in names) <= 64 << 20
+    out = {n[:-4]: np.load(tmp_path / 'a' / n) for n in names}
+    for n in names:
+        assert out[n[:-4]].dtype == np.float64 and np.array_equal(out[n[:-4]], np.load(tmp_path / 'b' / n))
+    idx = out['index'].astype(np.int64)
+    assert (len(idx) == n_mu) == (n_mu * n_red * 8 < bench.DUMP_BYTES) and np.all(np.diff(idx) > 0)
+    assert np.array_equal(out['u'], u.numpy()[idx]) and np.array_equal(out['mu'], mus[idx])
+    assert np.array_equal(out['eta'], mus[idx] ** 2) and not out['info'].any()
+    assert list(out['eta_max']) == [1.0, n_mu - 1]
+
+
 def test_synthetic_3d_fixture_structure():
     """The seeded synthetic operator set with 3D structure (config C4 shape): symmetry and definiteness where the hot path
     relies on them, interface-only coupling blocks, six-neighbour subdomain graph, determinism by seed."""
