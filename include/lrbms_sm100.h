@@ -185,7 +185,8 @@ int lrbms_plan_destroy(lrbms_plan_t plan);
 /* what: 0 = kernel launches per run, 1 = CTAs of the main kernel, 2 = algorithmic bytes per run (tight count),
  *       3 = algorithmic flops per run, 4 = device bytes owned by the plan, 5 = algorithmic bytes (SURVEY formula);
  *       online plans: 6 = solve kernel the plan selected (LRBMS_SOLVER_*), 7 = factor flops per parameter that kernel
- *       executes, 8 = scalar half bandwidth of the reduced operator */
+ *       executes, 8 = scalar half bandwidth of the reduced operator, 9 = parameters per CTA of the estimator kernel
+ *       (64, 32, 16 or 8; 0 without estimator terms) */
 int lrbms_plan_info(lrbms_plan_t plan, int32_t what, double* out);
 
 /* ---------------------------------------------------------------------------------------------------- */

@@ -43,10 +43,23 @@ struct lrbms_plan {
   size_t device_bytes = 0;
   double info_launches = 0, info_ctas = 0, info_bytes = 0, info_flops = 0, info_bytes_survey = 0;
   double info_solver = 0, info_solve_flops = 0, info_half_bandwidth = 0;   // online plans only
+  double info_est_tmu = 0;            // online plans with an estimator: parameters per estimator CTA
   virtual ~lrbms_plan() {}
   virtual int run(void* stream) = 0;
   virtual void ensure_info() {}       // byte / flop accounting is computed on first request, not at plan creation
 };
+
+// Opens a kernel's dynamic shared-memory limit to all the device allows one block beside the kernel's own static shared
+// memory, and returns that static size. The limit is an attribute of the function on the current device, shared by every
+// plan: set to one plan's byte count, it would make the next launch of a larger plan that is still alive fail. It does not
+// change occupancy, which follows the bytes a launch asks for.
+inline cudaError_t lrbms_open_dynamic_smem(const lrbms_context* ctx, const void* fn, size_t* static_bytes = nullptr) {
+  cudaFuncAttributes fa;
+  cudaError_t e = cudaFuncGetAttributes(&fa, fn);
+  if (e != cudaSuccess) return e;
+  if (static_bytes) *static_bytes = fa.sharedSizeBytes;
+  return cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->max_smem_optin - (int)fa.sharedSizeBytes);
+}
 
 extern thread_local std::string g_create_error;
 

@@ -149,6 +149,7 @@ int lrbms_plan_info(lrbms_plan_t plan, int32_t what, double* out) {
     case 6: *out = plan->info_solver; break;
     case 7: *out = plan->info_solve_flops; break;
     case 8: *out = plan->info_half_bandwidth; break;
+    case 9: *out = plan->info_est_tmu; break;
     default: return lrbms_fail(plan->ctx, LRBMS_ERR_INVALID, "lrbms_plan_info: unknown selector");
   }
   return LRBMS_OK;

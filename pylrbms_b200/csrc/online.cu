@@ -1137,12 +1137,12 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
 
   P->solve_smem = sizeof(double) * ((size_t)S.n_pad + 64 + 64 + kSolveWarps * 8 + sp.n_theta);
   if (sys->solver == LRBMS_SOLVER_GLOBAL_TILES) {
-    if (P->solve_smem > (size_t)h->max_smem_optin) {
+    size_t static1 = 0;
+    PLAN_CUDA_CHECK(lrbms_open_dynamic_smem(h, (const void*)solve_kernel, &static1));
+    if (P->solve_smem + static1 > (size_t)h->max_smem_optin) {
       lrbms_plan_destroy(P);
       return lrbms_fail(h, LRBMS_ERR_UNSUPPORTED, "online_plan_create: reduced dimension too large for the shared-memory solve vector");
     }
-    if (P->solve_smem > 48 * 1024)
-      PLAN_CUDA_CHECK(cudaFuncSetAttribute(solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P->solve_smem));
     int per_sm = 0;
     PLAN_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, solve_kernel, kSolveThreads, P->solve_smem));
     if (per_sm < 1) per_sm = 1;
@@ -1223,10 +1223,10 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
                                            (size_t)kABufs * mac * Q * 64) +
                          16 * ((size_t)kMetaBufs * MT + (size_t)(S.ntc + 1) + 2 * (size_t)S.ntc) + 8 * (size_t)kMetaBufs * mcp +
                          4 * (3 * (size_t)kMetaBufs * MT + S.ca_tile.size()) + 64;
-    cudaFuncAttributes fa2;
-    PLAN_CUDA_CHECK(cudaFuncGetAttributes(&fa2, solve_kernel_v2));
+    size_t static2 = 0;
+    PLAN_CUDA_CHECK(lrbms_open_dynamic_smem(h, (const void*)solve_kernel_v2, &static2));
     // the static shared memory of the kernel (mbarriers, status word) counts against the same per-block limit
-    if (bytes + fa2.sharedSizeBytes <= (size_t)h->max_smem_optin && sys->solver != LRBMS_SOLVER_GLOBAL_TILES &&
+    if (bytes + static2 <= (size_t)h->max_smem_optin && sys->solver != LRBMS_SOLVER_GLOBAL_TILES &&
         sys->solver != LRBMS_SOLVER_BANDED && sys->solver != LRBMS_SOLVER_PANEL) {
       SolveParamsV2& s2 = P->sp2;
       s2.base = sp;
@@ -1259,7 +1259,6 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
       }
 #endif
       P->solve2_smem = bytes;
-      PLAN_CUDA_CHECK(cudaFuncSetAttribute(solve_kernel_v2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
       P->use_v2 = true;
       P->solve_grid = h->sm_count;
       P->solve_stride = s2.base.work_stride;
@@ -1348,20 +1347,29 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
     auto est_bytes = [&](int tmu) {
       return sizeof(double) * ((size_t)(ep.dmax_pad + ep.qdmax_pad + 8) * (tmu + 4) + (size_t)Q * tmu + kEstWarps * 3 * tmu);
     };
+    // dynamic bytes each instantiation may ask for: the per-block limit minus its static shared memory (s_tile_ptr)
+    auto est_room = [&](int tmu, size_t* room) {
+      const void* fn = tmu == 64 ? (const void*)estimate_kernel<64>
+                       : tmu == 32 ? (const void*)estimate_kernel<32>
+                       : tmu == 16 ? (const void*)estimate_kernel<16> : (const void*)estimate_kernel<8>;
+      size_t st = 0;
+      const cudaError_t e = lrbms_open_dynamic_smem(h, fn, &st);
+      *room = (size_t)h->max_smem_optin - st;
+      return e;
+    };
     // 32 parameters per CTA when two such CTAs fit one SM (the staging phase of one overlaps the DMMAs of the other:
     // 4.5 instead of 5.4 ms per 10 000 parameters at C2), else the largest tile that fits at all
     P->est_tmu = (2 * (est_bytes(32) + 1024) <= (size_t)h->max_smem_optin) ? 32 : kTMUMax;
-    while (P->est_tmu > 8 && est_bytes(P->est_tmu) > (size_t)h->max_smem_optin) P->est_tmu /= 2;
+    size_t room = 0;
+    PLAN_CUDA_CHECK(est_room(P->est_tmu, &room));
+    while (P->est_tmu > 8 && est_bytes(P->est_tmu) > room) {
+      P->est_tmu /= 2;
+      PLAN_CUDA_CHECK(est_room(P->est_tmu, &room));
+    }
     P->est_smem = est_bytes(P->est_tmu);
-    if (P->est_smem > (size_t)h->max_smem_optin) {
+    if (P->est_smem > room) {
       lrbms_plan_destroy(P);
       return lrbms_fail(h, LRBMS_ERR_UNSUPPORTED, "online_plan_create: neighbourhood too large for the estimator kernel's shared memory");
-    }
-    if (P->est_smem > 48 * 1024) {
-      const void* fn = P->est_tmu == 64 ? (const void*)estimate_kernel<64>
-                       : P->est_tmu == 32 ? (const void*)estimate_kernel<32>
-                       : P->est_tmu == 16 ? (const void*)estimate_kernel<16> : (const void*)estimate_kernel<8>;
-      PLAN_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P->est_smem));
     }
     CombineParams& cp = P->cp;
     cp.n_sub = S.n_sub; cp.Q = Q; cp.n_theta = Q + Qf; cp.alpha_first = sys->alpha_returns_first;
@@ -1372,10 +1380,12 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
   P->info_launches = P->use_band ? 4.0 * P->band.nbc + 4 : 3;
   P->info_ctas = P->solve_grid;
   // introspection (lrbms_plan_info 6 .. 9): which solve kernel the plan selected, executed factor flops per parameter
-  // (the 8x8-tile count for the CTA-per-parameter kernels, the dense-band count of the band solver), half bandwidth
+  // (the 8x8-tile count for the CTA-per-parameter kernels, the dense-band count of the band solver), half bandwidth,
+  // parameters per estimator CTA
   P->info_solver = P->use_v3 ? LRBMS_SOLVER_PANEL : P->use_v2 ? LRBMS_SOLVER_WINDOW : P->use_band ? LRBMS_SOLVER_BANDED : LRBMS_SOLVER_GLOBAL_TILES;
   P->info_solve_flops = P->use_band ? P->band.flops_per_mu : P->use_v3 ? (double)P->sym3.flops : (double)S.flops;
   P->info_half_bandwidth = S.half_bandwidth;
+  P->info_est_tmu = P->has_estimator ? P->est_tmu : 0;
   // uploads and clears above ran on the legacy default stream: finish them before a caller's non-blocking stream runs the plan
   PLAN_CUDA_CHECK(cudaStreamSynchronize((cudaStream_t)0));
   *out = P;

@@ -581,12 +581,10 @@ size_t lrbms_v3_smem_bytes(const V3Params& P) {
 
 int lrbms_v3_prepare(lrbms_context* ctx, const V3Params& P, size_t* smem_out) {
   const size_t bytes = lrbms_v3_smem_bytes(P);
-  cudaFuncAttributes fa;
-  cudaError_t e = cudaFuncGetAttributes(&fa, solve_kernel_v3);
+  size_t static_bytes = 0;
+  cudaError_t e = lrbms_open_dynamic_smem(ctx, (const void*)solve_kernel_v3, &static_bytes);
   if (e != cudaSuccess) return lrbms_fail(ctx, LRBMS_ERR_CUDA, cudaGetErrorString(e));
-  if (bytes + fa.sharedSizeBytes > (size_t)ctx->max_smem_optin) return LRBMS_ERR_UNSUPPORTED;      // caller falls back
-  e = cudaFuncSetAttribute(solve_kernel_v3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) return lrbms_fail(ctx, LRBMS_ERR_CUDA, cudaGetErrorString(e));
+  if (bytes + static_bytes > (size_t)ctx->max_smem_optin) return LRBMS_ERR_UNSUPPORTED;      // caller falls back
   *smem_out = bytes;
   return LRBMS_OK;
 }

@@ -108,8 +108,7 @@ def test_c3_spe10_contrast_16x16(handle):
     rhs_ref = unblock(O.project_system(d_ref.rhs, red_ref.bases, red_ref.bases))
     lo, hi = data.parameter_range
     mus = np.linspace(lo, hi, 8)
-    U, eta = rd.sweep(mus)
-    assert np.all(np.isfinite(eta)) and np.all(eta > 0)
+    U, eta, parts, ind = rd.sweep(mus, decompose=True)
     for k, mu in enumerate(mus):
         mu_p = rd.parse_parameter(mu)
         A = np.asarray(op_ref.assemble(mu_p).matrix)
@@ -118,6 +117,48 @@ def test_c3_spe10_contrast_16x16(handle):
         e = U.data[k] - u_ref
         assert np.sqrt(e @ A @ e) <= RTOL * np.sqrt(u_ref @ A @ u_ref), 'mu {}'.format(mu)
     print('C3 (16x16) worst block rel err', worst)
+    # the estimator on all 256 subdomains against the exact value of the GPU's own reduced operators and u, and the
+    # estimator constants against the oracle's: with the blocks and solutions above this closes the chain to eta
+    _check_estimator(rd, mus, U, eta, parts, ind, range(data.num_subdomains), 'C3 (16x16)')
+    est, est_ref = rd.estimator, d_ref.estimator
+    rf2_ref = np.asarray(est_ref.local_eta_rf_squared, dtype=np.float64)
+    assert np.all(np.abs(est.local_eta_rf_squared - rf2_ref) <= 1e-13 * np.abs(rf2_ref))
+    rs_ref = (1.0 / np.pi ** 2) / np.asarray(est_ref.min_diffusion_evs) * np.asarray(est_ref.subdomain_diameters) ** 2
+    assert np.all(np.abs(est.r_scale() - rs_ref) <= 1e-15 * rs_ref)
+    for mu in mus:
+        mu_p, mu_r = rd.parse_parameter(mu), d_ref.parse_parameter(mu)
+        for f in ('alpha', 'gamma'):
+            for bar, bar_ref in ((est.mu_bar, est_ref.mu_bar), (est.mu_hat, est_ref.mu_hat)):
+                got = getattr(est, f)(est.lambda_coeffs, mu_p, bar)
+                ref = getattr(est_ref, f)(est_ref.lambda_coeffs, mu_r, bar_ref)
+                assert abs(got - ref) <= 1e-15 * abs(ref), (f, mu)
+
+
+def _check_estimator(rd, mus, U, eta, parts, ind, subdomains, what):
+    """The parts of ``rd.sweep(decompose=True)`` on ``subdomains`` within the kernel's rounding bound gamma_K S of their exact
+    value (oracle/exact_forms.py, tests/test_gpu_estimator.py); eta and the indicators of every subdomain as the float64
+    combine of the kernel's own parts (estimators.py:99-109)."""
+    from test_gpu_estimator import EPS, PARTS, gamma, model_K, model_exact
+    subs = list(subdomains)
+    forms, ex = model_exact(rd, mus, U.data, subs)
+    K = model_K(rd, forms, subs)
+    worst = {}
+    for k, name in enumerate(PARTS):
+        got = np.asarray(parts[k])[subs]
+        err = np.abs(got - ex[name])
+        assert np.all(err <= gamma(K[k][:, None]) * ex['S_' + name]), name
+        worst[name] = float((err / (EPS * ex['S_' + name])).max())
+    est = rd.estimator
+    nc, rdf = np.asarray(parts[0]), np.asarray(parts[1]) + np.asarray(parts[2])
+    for k, mu in enumerate(mus):
+        mu_p = rd.parse_parameter(mu)
+        lam = est.lambda_coeffs
+        a_bar, g_bar, a_hat = est.alpha(lam, mu_p, est.mu_bar), est.gamma(lam, mu_p, est.mu_bar), est.alpha(lam, mu_p, est.mu_hat)
+        e = (np.sqrt(g_bar) * np.sqrt(np.sum(nc[:, k] ** 2)) + np.sqrt(np.sum(rdf[:, k] ** 2)) / np.sqrt(a_hat)) / np.sqrt(a_bar)
+        assert abs(eta[k] - e) <= 8 * EPS * e
+        i_ref = (2.0 / a_bar) * (g_bar * nc[:, k] ** 2 + (1.0 / a_hat) * rdf[:, k] ** 2)
+        assert np.all(np.abs(np.asarray(ind)[:, k] - i_ref) <= 8 * EPS * np.abs(i_ref))
+    print(what, 'estimator |got - exact| / (eps S):', worst)
 
 
 def test_published_indicator_norms_cuda(handle):
@@ -150,7 +191,7 @@ def test_c4_3d_8x8x8_N40_full_size_online(handle):
     at FULL size on the band solver.  The reference's dense path cannot run here (one unblocked operator is 3.4 GB and it
     stores hundreds), so the check is against an independent CPU solver on the same block-sparse reduced operator
     (SciPy's SuperLU): energy-norm error and residual at 1e-10, plus bit-identical results for a different batch composition.
-    The estimator at this neighbourhood size (seven members, N = 40) is checked against the oracle in test_gpu_parity.py."""
+    The estimator runs on 17 parameters and is held to the exact value of its forms on a sample of 16 subdomains."""
     import scipy.sparse as sp
     import scipy.sparse.linalg as spl
     from pylrbms_b200 import LRBMSReductor, discretize
@@ -161,9 +202,18 @@ def test_c4_3d_8x8x8_N40_full_size_online(handle):
     rd = LRBMSReductor(discretize(data)[0], bases={'domain_%d' % i: bases[i] for i in range(S)}).reduce()
     assert rd.n_red == 20480 and rd.solve_kernel_name == 'band_update_kernel' and rd.half_bandwidth == 2599
     lo, hi = data.parameter_range
-    mus = np.array([lo, 0.5 * (lo + hi), hi])
-    U, eta = rd.sweep(mus)
-    assert np.all(np.isfinite(eta)) and np.all(eta > 0)
+    # 17 parameters: the estimator runs 16 per CTA here (seven-member neighbourhoods of 280 dofs), so two tiles
+    mus17 = np.linspace(lo, hi, 17)
+    U17, eta17, parts, ind = rd.sweep(mus17, decompose=True)
+    assert int(rd.online_plan.info(9)) == 16
+    # a sample of subdomains: corners, edges, faces, interior (seven-member neighbourhoods)
+    at = lambda x, y, z: (z * 8 + y) * 8 + x
+    sample = [at(0, 0, 0), at(7, 7, 7), at(7, 0, 0), at(0, 7, 7), at(3, 0, 0), at(0, 4, 7), at(7, 5, 0), at(2, 7, 7),
+              at(0, 3, 4), at(4, 0, 5), at(5, 6, 7), at(7, 2, 3), at(3, 3, 3), at(4, 4, 4), at(1, 6, 2), at(5, 2, 6)]
+    _check_estimator(rd, mus17, U17, eta17, parts, ind, sample, 'C4 (8x8x8)')
+    pick = [0, 8, 16]
+    mus = mus17[pick]
+    Ud, eta = np.asarray(U17.data)[pick], eta17[pick]
     # the block-sparse reduced operator on the host
     offs = np.concatenate([[0], np.cumsum(rd.block_dims)])
     mats = []
@@ -181,8 +231,8 @@ def test_c4_3d_8x8x8_N40_full_size_online(handle):
         lu = spl.splu(A)
         u_ref = lu.solve(f)
         u_ref += lu.solve(f - A @ u_ref)                                # one step of refinement on the CPU side
-        e = U.data[k] - u_ref
+        e = Ud[k] - u_ref
         assert np.sqrt(e @ (A @ e)) <= RTOL * np.sqrt(u_ref @ (A @ u_ref))
-        assert np.linalg.norm(A @ U.data[k] - f) <= RTOL * np.linalg.norm(f) * 100
+        assert np.linalg.norm(A @ Ud[k] - f) <= RTOL * np.linalg.norm(f) * 100
     U2, eta2 = rd.sweep(mus[[2, 0]])
-    assert np.array_equal(U2.data[0], U.data[2]) and np.array_equal(U2.data[1], U.data[0]) and eta2[0] == eta[2]
+    assert np.array_equal(U2.data[0], Ud[2]) and np.array_equal(U2.data[1], Ud[0]) and eta2[0] == eta[2]
