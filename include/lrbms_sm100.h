@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define LRBMS_VERSION 100
+#define LRBMS_VERSION 101
 
 typedef enum {
   LRBMS_OK = 0,
@@ -184,9 +184,9 @@ int lrbms_plan_run(lrbms_plan_t plan, void* stream);
 int lrbms_plan_destroy(lrbms_plan_t plan);
 /* what: 0 = kernel launches per run, 1 = CTAs of the main kernel, 2 = algorithmic bytes per run (tight count),
  *       3 = algorithmic flops per run, 4 = device bytes owned by the plan, 5 = algorithmic bytes (SURVEY formula);
- *       online plans: 6 = solve kernel the plan selected (LRBMS_SOLVER_*), 7 = factor flops per parameter that kernel
- *       executes, 8 = scalar half bandwidth of the reduced operator, 9 = parameters per CTA of the estimator kernel
- *       (64, 32, 16 or 8; 0 without estimator terms) */
+ *       online plans: 6 = solve kernel the plan selected (LRBMS_SOLVER_WINDOW or LRBMS_SOLVER_BANDED), 7 = factor flops
+ *       per parameter that kernel executes, 8 = scalar half bandwidth of the reduced operator, 9 = parameters per CTA of
+ *       the estimator kernel (64, 32, 16 or 8; 0 without estimator terms) */
 int lrbms_plan_info(lrbms_plan_t plan, int32_t what, double* out);
 
 /* ---------------------------------------------------------------------------------------------------- */
@@ -211,17 +211,6 @@ int lrbms_symbolic_info(lrbms_symbolic_t s, int32_t what, int64_t* out);
  * returns number of int32 written (<= cap) or a negative status */
 int64_t lrbms_symbolic_get(lrbms_symbolic_t s, int32_t which, int32_t* out, int64_t cap);
 
-/* Panel schedule of the two-column shared-memory kernel (solve_kernel_v3), built from a tile schedule; host-only.  Exposed so
- * that tests can execute the tables on the CPU.  info: 0 schedule applies (1) or not (0), 1 panels, 2 window slots, 3
- * accumulator rows, 4 partial blocks, 5 tiles of the closed pattern, 6 DMMA flops per parameter, 7 / 8 int32 words per
- * owner / panel record, 9 steps.  get: 0 col_ptr, 1 row_idx, 2 a_map, 3 win_slot, 4 owner records, 5 panel records, 6 steps
- * (record layouts: csrc/symbolic3.h). */
-typedef struct lrbms_symbolic3* lrbms_symbolic3_t;
-int lrbms_symbolic3_create(lrbms_symbolic_t s, lrbms_symbolic3_t* out);
-int lrbms_symbolic3_destroy(lrbms_symbolic3_t s);
-int lrbms_symbolic3_info(lrbms_symbolic3_t s, int32_t what, int64_t* out);
-int64_t lrbms_symbolic3_get(lrbms_symbolic3_t s, int32_t which, int32_t* out, int64_t cap);
-
 /* one estimator term:  out[kind][sub][mu] += coef * theta[qa](mu) * theta[qb](mu) * xl^T M xr  */
 enum { LRBMS_VEC_ONE = 0, LRBMS_VEC_UI = 1, LRBMS_VEC_UN = 2, LRBMS_VEC_UR = 3 };
 enum { LRBMS_OUT_NC = 0, LRBMS_OUT_R = 1, LRBMS_OUT_DF = 2 };
@@ -236,13 +225,11 @@ typedef struct {
   int64_t matrix_offset;   /* into the estimator matrix buffer, in doubles; M row-major, ld = cols */
 } lrbms_estimator_term_t;
 
-/* Solve kernel of an online plan.  AUTO: a shared-memory-window kernel (one SM per parameter, live factor window in
- * shared memory) when the window fits -- PANEL (two tile columns per pipeline stage, 2 x 2 register-blocked updates) when its
- * schedule applies, else WINDOW (one column per stage) -- else the block-banded out-of-HBM Cholesky (whole GPU per chunk).
- * WINDOW / BANDED force one of them (WINDOW fails with LRBMS_ERR_UNSUPPORTED when the window does not fit);
- * GLOBAL_TILES is the first-generation kernel (tile factor in global scratch), kept for cross-checks. */
-enum { LRBMS_SOLVER_AUTO = 0, LRBMS_SOLVER_WINDOW = 1, LRBMS_SOLVER_GLOBAL_TILES = 2, LRBMS_SOLVER_BANDED = 3,
-       LRBMS_SOLVER_PANEL = 4 };
+/* Solve kernel of an online plan.  AUTO: WINDOW, the shared-memory-window kernel (one SM per parameter, live factor window
+ * in shared memory), when the window fits one SM, else BANDED, the block-banded out-of-HBM Cholesky (whole GPU per chunk).
+ * WINDOW / BANDED force one of them (WINDOW fails with LRBMS_ERR_UNSUPPORTED when the window does not fit).  Any other
+ * value fails with LRBMS_ERR_INVALID. */
+enum { LRBMS_SOLVER_AUTO = 0, LRBMS_SOLVER_WINDOW = 1, LRBMS_SOLVER_BANDED = 3 };
 
 typedef struct {
   int32_t n_sub;

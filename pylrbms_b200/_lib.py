@@ -21,7 +21,6 @@ EXPORTS = [
     'lrbms_spmm_plan_create', 'lrbms_project_plan_create', 'lrbms_project_plan_scratch_bytes',
     'lrbms_project_plan_create_ws', 'lrbms_plan_run', 'lrbms_plan_destroy', 'lrbms_plan_info',
     'lrbms_symbolic_create', 'lrbms_symbolic_destroy', 'lrbms_symbolic_info', 'lrbms_symbolic_get',
-    'lrbms_symbolic3_create', 'lrbms_symbolic3_destroy', 'lrbms_symbolic3_info', 'lrbms_symbolic3_get',
     'lrbms_online_plan_create', 'lrbms_online_workspace_bytes', 'lrbms_online_solve', 'lrbms_online_estimate',
     'lrbms_online_sweep', 'lrbms_eta_max', 'lrbms_online_debug_timing',
     'lrbms_pcg_workspace_bytes', 'lrbms_pcg_solve', 'lrbms_remap_blocks', 'lrbms_peer_push',
@@ -29,8 +28,8 @@ EXPORTS = [
 
 VEC_ONE, VEC_UI, VEC_UN, VEC_UR = 0, 1, 2, 3
 OUT_NC, OUT_R, OUT_DF = 0, 1, 2
-SOLVER_AUTO, SOLVER_WINDOW, SOLVER_GLOBAL_TILES, SOLVER_BANDED, SOLVER_PANEL = 0, 1, 2, 3, 4
-SOLVER_NAMES = {1: 'solve_kernel_v2', 2: 'solve_kernel', 3: 'band_update_kernel', 4: 'solve_kernel_v3'}
+SOLVER_AUTO, SOLVER_WINDOW, SOLVER_BANDED = 0, 1, 3
+SOLVER_NAMES = {1: 'solve_kernel_v2', 3: 'band_update_kernel'}
 
 
 class LrbmsError(RuntimeError):
@@ -117,10 +116,6 @@ def load_library():
             'lrbms_symbolic_destroy': (C.c_int, [vp]),
             'lrbms_symbolic_info': (C.c_int, [vp, i32, P(i64)]),
             'lrbms_symbolic_get': (i64, [vp, i32, vp, i64]),
-            'lrbms_symbolic3_create': (C.c_int, [vp, P(vp)]),
-            'lrbms_symbolic3_destroy': (C.c_int, [vp]),
-            'lrbms_symbolic3_info': (C.c_int, [vp, i32, P(i64)]),
-            'lrbms_symbolic3_get': (i64, [vp, i32, vp, i64]),
             'lrbms_online_plan_create': (C.c_int, [vp, vp, P(vp)]),
             'lrbms_online_workspace_bytes': (C.c_int, [vp, i64, P(C.c_size_t)]),
             'lrbms_online_solve': (C.c_int, [vp, i64, vp, vp, vp, vp, C.c_size_t, vp]),

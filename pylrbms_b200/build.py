@@ -14,7 +14,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'liblrbms_sm100.so')
-SOURCES = ['context.cu', 'project.cu', 'online.cu', 'online3.cu', 'band.cu', 'pcg.cu', 'symbolic.cpp', 'symbolic3.cpp']
+SOURCES = ['context.cu', 'project.cu', 'online.cu', 'band.cu', 'pcg.cu', 'symbolic.cpp']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '-Xcompiler', '-fPIC',
               '-Xcompiler', '-fvisibility=default']
 if os.environ.get('LRBMS_DEVTOOLS', '0') not in ('', '0'):

@@ -1,13 +1,13 @@
 // Online half of the LRBMS hot path: mu-batched assembly + sparse Cholesky + solves of the block-sparse reduced
 // system (K3 + K4), mu-batched estimator quadratic forms (K5) and the eta combine / max reduction.
 //
-// solve_kernel: one CTA per parameter (grid-stride over the batch).  The reduced matrix lives as 8x8 tiles (the
-// DMMA.8x8x4 accumulator shape); the host-side symbolic phase (symbolic.cpp) provides, per tile of L, the list of
-// (L_IK, L_JK) pairs to subtract.  Per tile column J:  phase A -- every warp forms its target tiles
-// A_IJ(mu) - sum_K L_IK L_JK^T in registers with DMMA (A_IJ(mu) = sum_q theta_q(mu) A_q is assembled on the fly,
-// left to right like LincombOperator.assemble), warp 0 factors the diagonal tile and inverts it;  phase B -- every
-// warp multiplies its tiles by L_JJ^{-T} (two DMMAs) and stores them.  The right-hand side rides along as one more
-// tile row (forward substitution fused into the factorisation); the backward substitution runs from shared memory.
+// solve_kernel_v2: one CTA per parameter (grid-stride over the batch).  The reduced matrix lives as 8x8 tiles (the
+// DMMA.8x8x4 accumulator shape); the host-side symbolic phase (symbolic.cpp) provides, per tile column, its targets and
+// their (L_IK, L_JK) update pairs as slots of a shared-memory window of live factor tiles.  Every target
+// A_IJ(mu) - sum_K L_IK L_JK^T is accumulated with DMMA (A_IJ(mu) = sum_q theta_q(mu) A_q is assembled on the fly, left
+// to right like LincombOperator.assemble), the diagonal tile is factored and inverted, and the off-diagonal tiles are
+// multiplied by L_JJ^{-T}.  The right-hand side rides along as one more tile row (forward substitution fused into the
+// factorisation).  Systems whose window does not fit one SM's shared memory go to the band solver (band.cu).
 //
 // estimate_kernel: one CTA per (subdomain, tile of 32 parameters).  Every quadratic form x_L^T M x_R of
 // reference estimators.py:71-85 is evaluated for 32 parameters at once as Y = M X_R on DMMA followed by a column dot
@@ -17,252 +17,12 @@
 
 #include "band.h"
 #include "common.cuh"
-#include "online3.h"
 #include "symbolic.h"
 
 namespace {
 
-constexpr int kSolveThreads = 256;
-constexpr int kSolveWarps = kSolveThreads / 32;
-constexpr int kMaxT = 4;   // targets per warp and round kept in registers
-
-struct SolveParams {
-  int32_t n_red, n_pad, ntc, n_tiles, Q, Qf, n_theta, n_a_tiles;
-  const int32_t* col_ptr;
-  const int32_t* row_idx;
-  const int32_t* pair_ptr;
-  const int32_t* pair_a;
-  const int32_t* pair_b;
-  const int32_t* a_map;
-  const double* a_tiles;   // [Q][n_a_tiles][64]
-  const double* rhs;       // [Qf][n_pad]
-  int64_t work_stride;     // doubles of scratch per CTA: (n_tiles + ntc) * 64 tiles + ntc * 64 inverse diagonal tiles
-};
-
-// target tile = A(mu) tile (or rhs row) minus its update pairs; result in DMMA accumulator layout
-__device__ __forceinline__ void form_target(const SolveParams& P, const double* __restrict__ sth, const double* L,
-                                            int slot, int J, int lane, double& c0, double& c1) {
-  const int g = lane >> 2, t = lane & 3;
-  c0 = 0.0;
-  c1 = 0.0;
-  if (slot < P.n_tiles) {
-    const int ai = P.a_map[slot];
-    if (ai >= 0) {
-      const double2* __restrict__ at = reinterpret_cast<const double2*>(P.a_tiles + (int64_t)ai * 64 + g * 8 + 2 * t);
-      const int64_t qs = (int64_t)P.n_a_tiles * 32;   // stride between affine terms in double2
-      double2 v = __ldg(at);
-      c0 = sth[0] * v.x;
-      c1 = sth[0] * v.y;
-      for (int q = 1; q < P.Q; ++q) {
-        v = __ldg(at + q * qs);
-        c0 += sth[q] * v.x;
-        c1 += sth[q] * v.y;
-      }
-    }
-  } else if (g == 0) {
-    // forward-solve row: f(mu)[8J + 2t .. +1] in row 0 of the tile
-    for (int q = 0; q < P.Qf; ++q) {
-      const double* f = P.rhs + (int64_t)q * P.n_pad + 8 * J + 2 * t;
-      c0 += sth[P.Q + q] * __ldg(f);
-      c1 += sth[P.Q + q] * __ldg(f + 1);
-    }
-  }
-  const int p0 = P.pair_ptr[slot], p1 = P.pair_ptr[slot + 1];
-  double n0 = 0.0, n1 = 0.0;   // second accumulator chain: halves the dependent-DMMA latency
-  const int off = g * 8 + t;
-  int p = p0;
-  for (; p + 1 < p1; p += 2) {
-    const double* a = L + (int64_t)P.pair_a[p] * 64 + off;
-    const double* b = L + (int64_t)P.pair_b[p] * 64 + off;
-    const double* a2 = L + (int64_t)P.pair_a[p + 1] * 64 + off;
-    const double* b2 = L + (int64_t)P.pair_b[p + 1] * 64 + off;
-    const double x0 = a[0], x1 = a[4], y0 = b[0], y1 = b[4];
-    const double z0 = a2[0], z1 = a2[4], w0 = b2[0], w1 = b2[4];
-    dmma884(c0, c1, -x0, y0);
-    dmma884(n0, n1, -z0, w0);
-    dmma884(c0, c1, -x1, y1);
-    dmma884(n0, n1, -z1, w1);
-  }
-  if (p < p1) {
-    const double* a = L + (int64_t)P.pair_a[p] * 64 + off;
-    const double* b = L + (int64_t)P.pair_b[p] * 64 + off;
-    const double x0 = a[0], x1 = a[4], y0 = b[0], y1 = b[4];
-    dmma884(c0, c1, -x0, y0);
-    dmma884(c0, c1, -x1, y1);
-  }
-  c0 += n0;
-  c1 += n1;
-}
-
-// X = C * W^T with C in accumulator layout and W = L_JJ^{-1} (row-major 8x8 in shared memory)
-__device__ __forceinline__ void apply_inverse_transpose(const double* __restrict__ sW, int lane, double c0, double c1,
-                                                        double& x0, double& x1) {
-  const int g = lane >> 2, t = lane & 3;
-  x0 = 0.0;
-  x1 = 0.0;
-#pragma unroll
-  for (int kk = 0; kk < 2; ++kk) {
-    const int src = (lane & ~3) | (2 * kk + (t >> 1));
-    const double v0 = __shfl_sync(0xffffffffu, c0, src);
-    const double v1 = __shfl_sync(0xffffffffu, c1, src);
-    const double a = (t & 1) ? v1 : v0;                 // C[g][4kk + t]
-    const double b = sW[g * 8 + 4 * kk + t];            // B[k = 4kk + t][n = g] = W[g][4kk + t]
-    dmma884(x0, x1, a, b);
-  }
-}
-
-__global__ void __launch_bounds__(kSolveThreads, 2)
-solve_kernel(SolveParams P, int64_t n_mu, const double* __restrict__ theta, double* __restrict__ u, int32_t* __restrict__ info,
-             double* __restrict__ work) {
-  extern __shared__ double smem[];
-  double* sx = smem;                      // n_pad: y, then the solution
-  double* sW = sx + P.n_pad;              // 64: inverse of the current diagonal tile
-  double* sS = sW + 64;                   // 64: scratch for the diagonal tile
-  double* sred = sS + 64;                 // kSolveWarps * 8
-  double* sth = sred + kSolveWarps * 8;   // n_theta
-  __shared__ int s_info;
-
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int g = lane >> 2, t = lane & 3;
-  double* L = work + (int64_t)blockIdx.x * P.work_stride;
-  double* Winv = L + (int64_t)(P.n_tiles + P.ntc) * 64;
-
-  for (int64_t mu = blockIdx.x; mu < n_mu; mu += gridDim.x) {
-    __syncthreads();
-    for (int q = threadIdx.x; q < P.n_theta; q += kSolveThreads) sth[q] = theta[mu * P.n_theta + q];
-    if (threadIdx.x == 0) s_info = 0;
-    __syncthreads();
-
-    for (int J = 0; J < P.ntc; ++J) {
-      const int cp0 = P.col_ptr[J], cp1 = P.col_ptr[J + 1];
-      const int n_off = cp1 - cp0 - 1 + 1;        // off-diagonal L targets + the rhs target
-      // ---- diagonal tile: warp 0
-      if (warp == 0) {
-        double c0, c1;
-        form_target(P, sth, L, cp0, J, lane, c0, c1);
-        sS[g * 8 + 2 * t] = c0;
-        sS[g * 8 + 2 * t + 1] = c1;
-        __syncwarp();
-        const int i = lane & 7;
-        double a[8], rinv[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) a[j] = sS[i * 8 + j];
-        int bad = 0;
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-          double akk = __shfl_sync(0xffffffffu, a[k], k);
-          if (8 * J + k >= P.n_red) akk = 1.0;                 // padding rows: identity
-          if (!(akk > 0.0)) { if (!bad) bad = 8 * J + k + 1; akk = 1.0; }
-          const double r = rsqrt(akk);
-          rinv[k] = r;
-          const double lik = ((i == k) ? akk : a[k]) * r;
-          a[k] = lik;
-#pragma unroll
-          for (int j = k + 1; j < 8; ++j) {
-            const double ljk = __shfl_sync(0xffffffffu, lik, j);
-            a[j] -= lik * ljk;
-          }
-        }
-        if (bad && lane == 0 && s_info == 0) s_info = bad;
-        __syncwarp();
-        if (lane < 8) {
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const double v = (j <= i) ? a[j] : 0.0;
-            sS[i * 8 + j] = v;
-            L[(int64_t)cp0 * 64 + i * 8 + j] = v;
-          }
-        }
-        __syncwarp();
-        // inverse: lane j computes column j of W = L^{-1} by forward substitution (uniform code, broadcast reads)
-        const int jc = lane & 7;
-        double w[8];
-#pragma unroll
-        for (int ii = 0; ii < 8; ++ii) {
-          double s = (ii == jc) ? 1.0 : 0.0;
-#pragma unroll
-          for (int k = 0; k < ii; ++k) s -= sS[ii * 8 + k] * w[k];
-          w[ii] = s * rinv[ii];
-        }
-        if (lane < 8) {
-#pragma unroll
-          for (int ii = 0; ii < 8; ++ii) {
-            sW[ii * 8 + jc] = w[ii];
-            Winv[(int64_t)J * 64 + ii * 8 + jc] = w[ii];
-          }
-        }
-      }
-      // ---- off-diagonal targets and the rhs row: warps 1..7, kMaxT per warp and round
-      for (int base = 0; base < n_off; base += (kSolveWarps - 1) * kMaxT) {
-        double c[kMaxT][2];
-        int slot[kMaxT];
-        if (warp > 0) {
-#pragma unroll
-          for (int i = 0; i < kMaxT; ++i) {
-            const int q = base + i * (kSolveWarps - 1) + (warp - 1);
-            slot[i] = -1;
-            if (q < n_off) {
-              slot[i] = (q < n_off - 1) ? (cp0 + 1 + q) : (P.n_tiles + J);
-              form_target(P, sth, L, slot[i], J, lane, c[i][0], c[i][1]);
-            }
-          }
-        }
-        __syncthreads();   // diagonal inverse ready (first round); all targets of this round formed
-        if (warp > 0) {
-#pragma unroll
-          for (int i = 0; i < kMaxT; ++i) {
-            if (slot[i] >= 0) {
-              double x0, x1;
-              apply_inverse_transpose(sW, lane, c[i][0], c[i][1], x0, x1);
-              *reinterpret_cast<double2*>(L + (int64_t)slot[i] * 64 + g * 8 + 2 * t) = make_double2(x0, x1);
-              if (slot[i] >= P.n_tiles && g == 0) { sx[8 * J + 2 * t] = x0; sx[8 * J + 2 * t + 1] = x1; }
-            }
-          }
-        }
-      }
-      __syncthreads();     // column J of L (and y_J) visible to everybody
-    }
-
-    // ---- backward substitution  L^T u = y,  columns right to left
-    for (int J = P.ntc - 1; J >= 0; --J) {
-      const int cp0 = P.col_ptr[J], cp1 = P.col_ptr[J + 1];
-      double s0 = 0.0, s1 = 0.0;
-      for (int p = cp0 + 1 + warp; p < cp1; p += kSolveWarps) {
-        const double2 l = *reinterpret_cast<const double2*>(L + (int64_t)p * 64 + g * 8 + 2 * t);
-        const double xv = sx[8 * P.row_idx[p] + g];
-        s0 += l.x * xv;
-        s1 += l.y * xv;
-      }
-#pragma unroll
-      for (int o = 4; o < 32; o <<= 1) {
-        s0 += __shfl_xor_sync(0xffffffffu, s0, o);
-        s1 += __shfl_xor_sync(0xffffffffu, s1, o);
-      }
-      if (g == 0) { sred[warp * 8 + 2 * t] = s0; sred[warp * 8 + 2 * t + 1] = s1; }
-      __syncthreads();
-      if (warp == 0) {
-        const int cidx = lane & 7;
-        double v = sx[8 * J + cidx];
-#pragma unroll
-        for (int w = 0; w < kSolveWarps; ++w) v -= sred[w * 8 + cidx];
-        // u_c = sum_k W[k][c] v_k
-        double acc = 0.0;
-#pragma unroll
-        for (int k = 0; k < 8; ++k) acc += Winv[(int64_t)J * 64 + k * 8 + cidx] * __shfl_sync(0xffffffffu, v, k);
-        if (lane < 8) sx[8 * J + cidx] = acc;
-      }
-      __syncthreads();
-    }
-    for (int i = threadIdx.x; i < P.n_red; i += kSolveThreads) u[mu * P.n_red + i] = sx[i];
-    if (threadIdx.x == 0 && info) info[mu] = s_info;
-  }
-}
-
 // ------------------------------------------------------------------------------------------------------
-//  solve_kernel_v2: the same left-looking 8x8-tile Cholesky, restructured around shared memory.
-//
-//  v1 keeps the factor of a parameter in global scratch and walks one dependent chain of L2-latency loads per tile
-//  column (ncu: tensor pipe 20 % active, 32 GB of DRAM traffic per 10 000 parameters).  v2:
+//  solve_kernel_v2: left-looking 8x8-tile Cholesky around shared memory.
 //    * one CTA of 16 warps per SM; the *live window* of L -- off-diagonal tiles (I, K) with K < J <= I, 253 tiles
 //      for the C2 band -- stays in shared memory in DMMA operand-fragment order (one conflict-free LDS.128 per lane
 //      and operand); the factor goes to global memory only once, for the backward substitution;
@@ -279,7 +39,11 @@ constexpr int kMetaBufs = 5;     // column metadata: columns J-1 .. J+3 are aliv
 constexpr int kABufs = 3;        // staged operator tiles: only needed while a column's early updates run
 
 struct SolveParamsV2 {
-  SolveParams base;
+  int32_t n_red, n_pad, Q, Qf, n_theta, n_a_tiles, ntc;
+  const int32_t* row_idx;   // [n_tiles] tile row of every factor slot
+  const double* a_tiles;    // [Q][n_a_tiles][64]
+  const double* rhs;        // [Qf][n_pad]
+  int64_t work_stride;      // doubles of factor scratch per CTA: n_tiles * 64
   const int4* ccol;         // [ntc + 1] {first tile, tiles, first item, tile (J+1, J) exists}
   const int4* ccol2;        // [ntc] {first tile pair, tile pairs, first rhs pair, rhs pairs}
   const int4* ccol3;        // [ntc] {first staged operator tile, staged operator tiles, 0, 0}
@@ -335,26 +99,25 @@ __device__ __forceinline__ void apply_pairs(const int2* __restrict__ pairs, cons
 }
 
 __global__ void __launch_bounds__(kV2Threads, 1)
-solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta, double* __restrict__ u,
+solve_kernel_v2(SolveParamsV2 P, int64_t n_mu, const double* __restrict__ theta, double* __restrict__ u,
                 int32_t* __restrict__ info, double* __restrict__ work) {
-  const SolveParams& P = P2.base;
   extern __shared__ __align__(16) double smem[];
-  const int MT = P2.max_targets;
+  const int MT = P.max_targets;
   double* win = smem;                                         // region_doubles
-  double* acc0 = win + P2.region_doubles;                     // 3 * MT * 64: target sums of columns J-1, J, J+1
+  double* acc0 = win + P.region_doubles;                      // 3 * MT * 64: target sums of columns J-1, J, J+1
   double* sx = acc0 + 3 * MT * 64;                            // n_pad
   double* sW = sx + P.n_pad;                                  // 2 * 64: L_JJ^{-1} of the current and the previous column
   double* sScr = sW + 2 * 64;                                 // 2 * 64: layout-conversion scratch (shared tile, chain warp)
   double* sred = sScr + 2 * 64;                               // 2 * kV2Warps * 8
   double* sth = sred + 2 * kV2Warps * 8;                      // n_theta (<= 32)
   double* sA = sth + 32;                                      // kABufs * max_a_col * Q * 64
-  const int a_buf_doubles = P2.max_a_col * P.Q * 64;
+  const int a_buf_doubles = P.max_a_col * P.Q * 64;
   int4* sDesc = reinterpret_cast<int4*>(sA + kABufs * a_buf_doubles);             // kMetaBufs * MT
   int4* sCol = sDesc + kMetaBufs * MT;                                            // ntc + 1
   int4* sCol2 = sCol + (P.ntc + 1);                                               // ntc
   int4* sCol3 = sCol2 + P.ntc;                                                    // ntc
   int2* sPair = reinterpret_cast<int2*>(sCol3 + P.ntc);                           // kMetaBufs * max_col_pairs
-  int* sSlot = reinterpret_cast<int*>(sPair + kMetaBufs * P2.max_col_pairs);      // kMetaBufs * MT
+  int* sSlot = reinterpret_cast<int*>(sPair + kMetaBufs * P.max_col_pairs);       // kMetaBufs * MT
   int* sOrd = sSlot + kMetaBufs * MT;                                             // kMetaBufs * MT
   int* sNext = sOrd + kMetaBufs * MT;                                             // kMetaBufs * MT
   int* sCaTile = sNext + kMetaBufs * MT;                                          // n_ca
@@ -365,7 +128,7 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
   const int g = lane >> 2, t = lane & 3;
   double* L = work + (int64_t)blockIdx.x * P.work_stride;
 #ifdef LRBMS_DEVTOOLS
-  const bool timing = P2.timing != nullptr && blockIdx.x == 0;
+  const bool timing = P.timing != nullptr && blockIdx.x == 0;
   long long tph[8] = {0, 0, 0, 0, 0, 0, 0, 0}, tlast = 0;
 // (bar.sync compiles to BAR.SYNC.DEFER_BLOCKING: a clock read right behind it is taken before the wait; the volatile
 // shared-memory read makes the barrier complete first)
@@ -375,9 +138,9 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
 #endif
 
   // ---- per-column tables: loaded once per CTA, no global-memory latency inside the column loop afterwards
-  for (int i = threadIdx.x; i <= P.ntc; i += kV2Threads) sCol[i] = P2.ccol[i];
-  for (int i = threadIdx.x; i < P.ntc; i += kV2Threads) { sCol2[i] = P2.ccol2[i]; sCol3[i] = P2.ccol3[i]; }
-  for (int i = threadIdx.x; i < P2.n_ca; i += kV2Threads) sCaTile[i] = P2.ca_tile[i];
+  for (int i = threadIdx.x; i <= P.ntc; i += kV2Threads) sCol[i] = P.ccol[i];
+  for (int i = threadIdx.x; i < P.ntc; i += kV2Threads) { sCol2[i] = P.ccol2[i]; sCol3[i] = P.ccol3[i]; }
+  for (int i = threadIdx.x; i < P.n_ca; i += kV2Threads) sCaTile[i] = P.ca_tile[i];
   __syncthreads();
 
   // stage everything column Jn needs into buffer Jn % kMetaBufs / Jn % kABufs.  Called by ONE producer warp (the
@@ -390,14 +153,14 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
       const int4 ci = sCol2[Jn];
       const int4 c3 = sCol3[Jn];
       for (int i = lane; i <= col.y; i += 32) {
-        cp_async16(sDesc + b * MT + i, P2.cdesc + col.z + i);
-        cp_async4(sSlot + b * MT + i, P2.cslot + col.z + i);
-        cp_async4(sOrd + b * MT + i, P2.cord + col.z + i);
-        cp_async4(sNext + b * MT + i, P2.cnext + col.z + i);
+        cp_async16(sDesc + b * MT + i, P.cdesc + col.z + i);
+        cp_async4(sSlot + b * MT + i, P.cslot + col.z + i);
+        cp_async4(sOrd + b * MT + i, P.cord + col.z + i);
+        cp_async4(sNext + b * MT + i, P.cnext + col.z + i);
       }
-      int2* dst = sPair + b * P2.max_col_pairs;
-      for (int i = lane; i < ci.y; i += 32) cp_async8(dst + i, P2.win_ab + ci.x + i);
-      for (int i = lane; i < ci.w; i += 32) cp_async8(dst + ci.y + i, P2.win_ab + ci.z + i);
+      int2* dst = sPair + b * P.max_col_pairs;
+      for (int i = lane; i < ci.y; i += 32) cp_async8(dst + i, P.win_ab + ci.x + i);
+      for (int i = lane; i < ci.w; i += 32) cp_async8(dst + ci.y + i, P.win_ab + ci.z + i);
       // raw operator tiles A_q of the column's targets (the theta-weighted sum is formed when they are consumed):
       // one 16-byte chunk per lane, 32 lanes = one tile per step
       double* adst = sA + (Jn % kABufs) * a_buf_doubles;
@@ -418,7 +181,7 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
   auto early_updates = [&](int Jx, double* accX) {
     const int mb = Jx % kMetaBufs;
     const int4* descC = sDesc + mb * MT;
-    const int2* pairC = sPair + mb * P2.max_col_pairs;
+    const int2* pairC = sPair + mb * P.max_col_pairs;
     const int* ordC = sOrd + mb * MT;
     const double* aC = sA + (Jx % kABufs) * a_buf_doubles;
     const int ncol = sCol[Jx].y;
@@ -479,7 +242,7 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
     const int mbn = (Jy + 1) % kMetaBufs;
     const int* slotN = sSlot + mbn * MT;
     const int4* descN = sDesc + mbn * MT;
-    const int2* pairN = sPair + mbn * P2.max_col_pairs;
+    const int2* pairN = sPair + mbn * P.max_col_pairs;
     const int ncolN = (Jy + 1 < P.ntc) ? sCol[Jy + 1].y : 0;
     double2 fbn = make_double2(0.0, 0.0);
     // Slot 0: L_{Jy+1,Jy} (every warp forms it itself instead of waiting for another warp); slots 1, 2: two of this
@@ -575,7 +338,7 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
       __syncwarp();
     }
     if (sSlot[(Jc % kMetaBufs) * MT] >> 20) {                                              // pair with source column Jc - 2
-      const int2 ab = sPair[(Jc % kMetaBufs) * P2.max_col_pairs + sDesc[(Jc % kMetaBufs) * MT].y];
+      const int2 ab = sPair[(Jc % kMetaBufs) * P.max_col_pairs + sDesc[(Jc % kMetaBufs) * MT].y];
       const double2 fa = *reinterpret_cast<const double2*>(win + ab.x * 64 + lane * 2);
       const double2 fb = *reinterpret_cast<const double2*>(win + ab.y * 64 + lane * 2);
       double2 cc = *reinterpret_cast<const double2*>(accCur + lane * 2);
@@ -657,7 +420,7 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
         diagonal_chain(J, accPrev, accCur, sWprev, sWcur);
         LRBMS_TICK(1);
       } else if (is_upd) {
-        if (P2.staggered) {
+        if (P.staggered) {
           // The early updates of column J+1 (source columns <= J-2) do not touch anything the triangular solve of column
           // J-1 produces, so the two run in either order: odd update warps solve first, even ones second -- the
           // bandwidth-bound pair loops of one half overlap the latency-bound solves of the other.
@@ -695,7 +458,7 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
     //                  earlier by the other warps), the one contribution that needs u_{J+1}, then L_JJ^{-T} -- while
     //                  warps 1..15 already form the partial sums of column J-1 from u_I, I >= J+1.  One barrier per column.
     {
-      const int stage = P2.back_stage_doubles;
+      const int stage = P.back_stage_doubles;
       auto issue = [&](int Jc) {
         if (Jc >= 0) {
           const int4 col = sCol[Jc];
@@ -796,7 +559,7 @@ solve_kernel_v2(SolveParamsV2 P2, int64_t n_mu, const double* __restrict__ theta
   }
 #ifdef LRBMS_DEVTOOLS
   if (timing && lane == 0)
-    for (int k = 0; k < 8; ++k) P2.timing[warp * 8 + k] = tph[k];
+    for (int k = 0; k < 8; ++k) P.timing[warp * 8 + k] = tph[k];
 #endif
 #undef LRBMS_TICK
 }
@@ -1015,17 +778,12 @@ __global__ void eta_max_kernel(int64_t n, const double* __restrict__ eta, double
 // ------------------------------------------------------------------------------------------------------
 struct OnlinePlan : lrbms_plan {
   lrbms_symbolic sym;
-  SolveParams sp;
+  // selected solve kernel: LRBMS_SOLVER_WINDOW (solve_kernel_v2) or LRBMS_SOLVER_BANDED (band.cu: block-banded
+  // out-of-HBM Cholesky for systems whose factor window exceeds one SM)
+  int solver = LRBMS_SOLVER_AUTO;
   SolveParamsV2 sp2;
-  bool use_v2 = false;
-  bool use_band = false;        // block-banded out-of-HBM Cholesky (band.cu): systems whose factor window exceeds one SM
   lrbms_band_plan band;
-  bool use_v3 = false;          // two-column panel kernel (online3.cu)
-  lrbms_symbolic3 sym3;
-  V3Params v3;
-  size_t v3_smem = 0;
-  size_t solve2_smem = 0;
-  int64_t solve_stride = 0;     // doubles of factor scratch per resident CTA of the selected solve kernel
+  int64_t solve_stride = 0;     // doubles of factor scratch per resident CTA of the window kernel
   EstParams ep;
   CombineParams cp;
   int solve_grid = 0;
@@ -1044,19 +802,19 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
   LRBMS_REQUIRE(h, h && sys && out, "online_plan_create: null argument");
   LRBMS_REQUIRE(h, sys->Q >= 1 && sys->Q <= 16 && sys->Qf >= 1 && sys->Qf <= 16, "online_plan_create: 1 <= Q, Qf <= 16");
   LRBMS_REQUIRE(h, sys->lhs_blocks && sys->rhs && sys->block_offset && sys->basis_sizes, "online_plan_create: null data pointer");
+  LRBMS_REQUIRE(h, sys->solver == LRBMS_SOLVER_AUTO || sys->solver == LRBMS_SOLVER_WINDOW || sys->solver == LRBMS_SOLVER_BANDED,
+                "online_plan_create: unknown solver");
   LRBMS_CUDA_CHECK(h, cudaSetDevice(h->device));
   OnlinePlan* P = new OnlinePlan();
   P->ctx = h;
   P->kind = PLAN_ONLINE;
   std::string err;
-  LRBMS_REQUIRE(h, sys->solver >= LRBMS_SOLVER_AUTO && sys->solver <= LRBMS_SOLVER_PANEL, "online_plan_create: unknown solver");
   int rc = lrbms_symbolic_basics(P->sym, sys->n_sub, sys->basis_sizes, sys->n_blocks, sys->block_i, sys->block_j, &err);
   if (rc) { delete P; return lrbms_fail(h, rc, err); }
-  // The 8x8-tile schedule is only built when a CTA-per-parameter kernel can use it: its pair lists grow like
+  // The 8x8-tile schedule is only built when the window kernel can use it: its pair lists grow like
   // n (b / 8)^2 / 2 (135 M pairs for the 8x8x8, N = 40 system), the band solver needs none of it.
   const double est_pairs = 0.5 * P->sym.ntc * (P->sym.half_bandwidth / 8.0 + 1.0) * (P->sym.half_bandwidth / 8.0 + 1.0);
-  bool tiles_built = sys->solver == LRBMS_SOLVER_WINDOW || sys->solver == LRBMS_SOLVER_GLOBAL_TILES || sys->solver == LRBMS_SOLVER_PANEL ||
-               (sys->solver == LRBMS_SOLVER_AUTO && est_pairs <= 3.0e7);
+  const bool tiles_built = sys->solver == LRBMS_SOLVER_WINDOW || (sys->solver == LRBMS_SOLVER_AUTO && est_pairs <= 3.0e7);
   if (tiles_built) {
     rc = lrbms_symbolic_build(P->sym, sys->n_sub, sys->basis_sizes, sys->n_blocks, sys->block_i, sys->block_j, &err);
     if (rc) { delete P; return lrbms_fail(h, rc, err); }
@@ -1121,100 +879,8 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
   double* d_f64 = nullptr;
 #define UP_I32(field, vec) do { rc = plan_upload(P, &d_i32, vec); if (rc) { lrbms_plan_destroy(P); return rc; } field = d_i32; } while (0)
 #define UP_F64(field, vec) do { rc = plan_upload(P, &d_f64, vec); if (rc) { lrbms_plan_destroy(P); return rc; } field = d_f64; } while (0)
-  SolveParams& sp = P->sp;
+  // ---- shared-memory-window kernel: used whenever the live window of L fits into the shared memory of one SM
   if (tiles_built) {
-  sp.n_red = S.n_red; sp.n_pad = S.n_pad; sp.ntc = S.ntc; sp.n_tiles = (int32_t)S.n_tiles(); sp.Q = Q; sp.Qf = Qf;
-  sp.n_theta = Q + Qf; sp.n_a_tiles = S.n_a_tiles;
-  sp.work_stride = ((int64_t)S.n_tiles() + 2 * S.ntc) * 64;
-  UP_I32(sp.col_ptr, S.col_ptr);
-  UP_I32(sp.row_idx, S.row_idx);
-  UP_I32(sp.pair_ptr, S.pair_ptr);
-  UP_I32(sp.pair_a, S.pair_a);
-  UP_I32(sp.pair_b, S.pair_b);
-  UP_I32(sp.a_map, S.a_map);
-  UP_F64(sp.a_tiles, tiles);
-  UP_F64(sp.rhs, rhs_h);
-
-  P->solve_smem = sizeof(double) * ((size_t)S.n_pad + 64 + 64 + kSolveWarps * 8 + sp.n_theta);
-  if (sys->solver == LRBMS_SOLVER_GLOBAL_TILES) {
-    size_t static1 = 0;
-    PLAN_CUDA_CHECK(lrbms_open_dynamic_smem(h, (const void*)solve_kernel, &static1));
-    if (P->solve_smem + static1 > (size_t)h->max_smem_optin) {
-      lrbms_plan_destroy(P);
-      return lrbms_fail(h, LRBMS_ERR_UNSUPPORTED, "online_plan_create: reduced dimension too large for the shared-memory solve vector");
-    }
-    int per_sm = 0;
-    PLAN_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, solve_kernel, kSolveThreads, P->solve_smem));
-    if (per_sm < 1) per_sm = 1;
-    P->solve_grid = per_sm * h->sm_count;
-  }
-  P->solve_stride = sp.work_stride;
-  // ---- two-column panel kernel (v3): on request only -- measured slower than the one-column kernel (profiles/README.md:
-  //      bound by warp 0's critical chain of two 8x8 Cholesky + inverses per panel), kept with its CPU-emulated schedule
-  if (sys->solver == LRBMS_SOLVER_PANEL) {
-    rc = lrbms_symbolic3_build(P->sym3, S);
-    if (rc) { lrbms_plan_destroy(P); return rc; }
-    const lrbms_symbolic3& S3 = P->sym3;
-    if (S3.ok) {
-      V3Params& v = P->v3;
-      int max_col = 1;
-      std::vector<int32_t> ccol(4 * (size_t)S3.ntc, 0);
-      for (int J = 0; J < S3.ntc; ++J) {
-        const int32_t c0 = S3.col_ptr[J], nc = S3.col_ptr[J + 1] - c0;
-        ccol[4 * J] = c0; ccol[4 * J + 1] = nc;
-        ccol[4 * J + 3] = (nc >= 2 && S3.row_idx[c0 + 1] == J + 1) ? 1 : 0;
-        max_col = std::max(max_col, nc);
-      }
-      v.n_red = S.n_red; v.n_pad = S.n_pad; v.ntc = S3.ntc; v.np = S3.np; v.Q = Q; v.Qf = Qf; v.n_theta = Q + Qf;
-      v.n_a_tiles = S.n_a_tiles; v.n_win = S3.n_win_slots; v.acc_rows = S3.acc_rows; v.n_partial = std::max(1, S3.n_partial);
-      v.max_col = max_col;
-      v.max_steps = std::max(1, S3.max_steps);
-      v.back_stage_doubles = max_col * 64;
-      v.region_doubles = std::max((S3.n_win_slots + 1) * 64, lrbms_v3_back_stages() * max_col * 64);
-      v.work_stride = S3.n_tiles() * 64;
-      v.a_tiles = sp.a_tiles; v.rhs = sp.rhs;
-      v.timing = nullptr;
-#ifdef LRBMS_DEVTOOLS
-      if (const char* tenv = getenv("LRBMS_SOLVE_TIMING")) {
-        if (atoi(tenv) > 0) {
-          rc = plan_alloc(P, &v.timing, (size_t)kV3Warps * 8);
-          if (rc) { lrbms_plan_destroy(P); return rc; }
-          PLAN_CUDA_CHECK(cudaMemset(v.timing, 0, sizeof(long long) * kV3Warps * 8));
-        }
-      }
-#endif
-      size_t smem3 = 0;
-      rc = lrbms_v3_prepare(h, v, &smem3);
-      if (rc == LRBMS_OK) {
-        std::vector<int32_t> steps = S3.steps;
-        if (steps.empty()) steps.assign(4, 0);
-        V3Own* d_own = nullptr; V3Panel* d_pan = nullptr;
-        rc = plan_upload(P, &d_own, S3.own);
-        if (!rc) rc = plan_upload(P, &d_pan, S3.pan);
-        if (rc) { lrbms_plan_destroy(P); return rc; }
-        v.own = d_own; v.pan = d_pan;
-        const int32_t* tmp = nullptr;
-        UP_I32(tmp, steps); v.steps = reinterpret_cast<const int4*>(tmp);
-        UP_I32(tmp, ccol);  v.ccol = reinterpret_cast<const int4*>(tmp);
-        UP_I32(v.row_idx, S3.row_idx);
-        P->v3_smem = smem3;
-        P->use_v3 = true;
-        P->solve_grid = h->sm_count;
-        P->solve_stride = v.work_stride;
-      } else if (rc != LRBMS_ERR_UNSUPPORTED) {
-        lrbms_plan_destroy(P);
-        return rc;
-      }
-    }
-  }
-  if (sys->solver == LRBMS_SOLVER_PANEL && !P->use_v3) {
-    const std::string why = "online_plan_create: the panel kernel does not apply (" +
-                            (P->sym3.why.empty() ? std::string("window does not fit") : P->sym3.why) + ")";
-    lrbms_plan_destroy(P);
-    return lrbms_fail(h, LRBMS_ERR_UNSUPPORTED, why);
-  }
-  // ---- shared-memory-window kernel (v2): used whenever the live window of L fits into shared memory
-  if (!P->use_v3) {
     const int maxcol = std::max(1, S.max_targets - 1);
     const int MT = S.max_targets;
     const int64_t region = std::max<int64_t>((int64_t)S.n_win_slots * 64, (int64_t)kBackStages * maxcol * 64);
@@ -1226,11 +892,14 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
     size_t static2 = 0;
     PLAN_CUDA_CHECK(lrbms_open_dynamic_smem(h, (const void*)solve_kernel_v2, &static2));
     // the static shared memory of the kernel (mbarriers, status word) counts against the same per-block limit
-    if (bytes + static2 <= (size_t)h->max_smem_optin && sys->solver != LRBMS_SOLVER_GLOBAL_TILES &&
-        sys->solver != LRBMS_SOLVER_BANDED && sys->solver != LRBMS_SOLVER_PANEL) {
+    if (bytes + static2 <= (size_t)h->max_smem_optin) {
       SolveParamsV2& s2 = P->sp2;
-      s2.base = sp;
-      s2.base.work_stride = (int64_t)S.n_tiles() * 64;
+      s2.n_red = S.n_red; s2.n_pad = S.n_pad; s2.ntc = S.ntc; s2.Q = Q; s2.Qf = Qf; s2.n_theta = Q + Qf;
+      s2.n_a_tiles = S.n_a_tiles;
+      s2.work_stride = (int64_t)S.n_tiles() * 64;
+      UP_I32(s2.row_idx, S.row_idx);
+      UP_F64(s2.a_tiles, tiles);
+      UP_F64(s2.rhs, rhs_h);
       s2.region_doubles = (int32_t)region;
       s2.max_targets = MT;
       s2.max_col_pairs = mcp;
@@ -1258,24 +927,22 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
         }
       }
 #endif
-      P->solve2_smem = bytes;
-      P->use_v2 = true;
+      P->solve_smem = bytes;
+      P->solver = LRBMS_SOLVER_WINDOW;
       P->solve_grid = h->sm_count;
-      P->solve_stride = s2.base.work_stride;
+      P->solve_stride = s2.work_stride;
     }
   }
-
-  }  // tiles_built
-  if (sys->solver == LRBMS_SOLVER_WINDOW && !P->use_v2) {
+  if (sys->solver == LRBMS_SOLVER_WINDOW && P->solver != LRBMS_SOLVER_WINDOW) {
     lrbms_plan_destroy(P);
     return lrbms_fail(h, LRBMS_ERR_UNSUPPORTED, "online_plan_create: the live factor window does not fit the shared memory of one SM");
   }
   // ---- band solver (band.cu): everything the CTA-per-parameter window kernel cannot hold
-  if (!P->use_v2 && !P->use_v3 && sys->solver != LRBMS_SOLVER_GLOBAL_TILES) {
+  if (P->solver != LRBMS_SOLVER_WINDOW) {
     rc = lrbms_band_build(P, P->band, S.n_sub, S.sizes.data(), S.offsets.data(), Q, Qf, sys->n_blocks, sys->block_i, sys->block_j,
                           sys->block_offset, hb.data(), tmp.data());
     if (rc) { lrbms_plan_destroy(P); return rc; }
-    P->use_band = true;
+    P->solver = LRBMS_SOLVER_BANDED;
     P->solve_grid = h->sm_count;
   }
 
@@ -1377,13 +1044,13 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
   }
 #undef UP_I32
 #undef UP_F64
-  P->info_launches = P->use_band ? 4.0 * P->band.nbc + 4 : 3;
+  P->info_launches = P->solver == LRBMS_SOLVER_BANDED ? 4.0 * P->band.nbc + 4 : 3;
   P->info_ctas = P->solve_grid;
   // introspection (lrbms_plan_info 6 .. 9): which solve kernel the plan selected, executed factor flops per parameter
-  // (the 8x8-tile count for the CTA-per-parameter kernels, the dense-band count of the band solver), half bandwidth,
+  // (the 8x8-tile count for the window kernel, the dense-band count of the band solver), half bandwidth,
   // parameters per estimator CTA
-  P->info_solver = P->use_v3 ? LRBMS_SOLVER_PANEL : P->use_v2 ? LRBMS_SOLVER_WINDOW : P->use_band ? LRBMS_SOLVER_BANDED : LRBMS_SOLVER_GLOBAL_TILES;
-  P->info_solve_flops = P->use_band ? P->band.flops_per_mu : P->use_v3 ? (double)P->sym3.flops : (double)S.flops;
+  P->info_solver = P->solver;
+  P->info_solve_flops = P->solver == LRBMS_SOLVER_BANDED ? P->band.flops_per_mu : (double)S.flops;
   P->info_half_bandwidth = S.half_bandwidth;
   P->info_est_tmu = P->has_estimator ? P->est_tmu : 0;
   // uploads and clears above ran on the legacy default stream: finish them before a caller's non-blocking stream runs the plan
@@ -1393,7 +1060,7 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
 }
 
 static size_t solve_ws_bytes(const OnlinePlan* P, int64_t n_mu) {
-  if (P->use_band) return lrbms_band_workspace_bytes(P->band, n_mu);
+  if (P->solver == LRBMS_SOLVER_BANDED) return lrbms_band_workspace_bytes(P->band, n_mu);
   const int64_t ctas = std::min<int64_t>(P->solve_grid, std::max<int64_t>(1, n_mu));
   return (size_t)ctas * P->solve_stride * sizeof(double);
 }
@@ -1414,7 +1081,7 @@ int lrbms_online_solve(lrbms_plan_t plan, int64_t n_mu, const double* theta, dou
   OnlinePlan* P = static_cast<OnlinePlan*>(plan);
   LRBMS_REQUIRE(P->ctx, theta && u && workspace, "online_solve: null argument");
   if (n_mu <= 0) return LRBMS_OK;
-  if (P->use_band) {
+  if (P->solver == LRBMS_SOLVER_BANDED) {
     // the band solver works through the batch in chunks of as many parameters as the workspace holds factors for
     LRBMS_REQUIRE(P->ctx, lrbms_band_chunk(P->band, n_mu, workspace_bytes) >= 1,
                   "online_solve: workspace too small (see lrbms_online_workspace_bytes)");
@@ -1423,12 +1090,7 @@ int lrbms_online_solve(lrbms_plan_t plan, int64_t n_mu, const double* theta, dou
   }
   LRBMS_REQUIRE(P->ctx, workspace_bytes >= solve_ws_bytes(P, n_mu), "online_solve: workspace too small (see lrbms_online_workspace_bytes)");
   const int grid = (int)std::min<int64_t>(P->solve_grid, n_mu);
-  if (P->use_v3)
-    lrbms_v3_launch(P->v3, grid, P->v3_smem, n_mu, theta, u, info, (double*)workspace, (cudaStream_t)stream);
-  else if (P->use_v2)
-    solve_kernel_v2<<<grid, kV2Threads, P->solve2_smem, (cudaStream_t)stream>>>(P->sp2, n_mu, theta, u, info, (double*)workspace);
-  else
-    solve_kernel<<<grid, kSolveThreads, P->solve_smem, (cudaStream_t)stream>>>(P->sp, n_mu, theta, u, info, (double*)workspace);
+  solve_kernel_v2<<<grid, kV2Threads, P->solve_smem, (cudaStream_t)stream>>>(P->sp2, n_mu, theta, u, info, (double*)workspace);
   LRBMS_CUDA_CHECK(P->ctx, cudaGetLastError());
   return LRBMS_OK;
 }
@@ -1469,7 +1131,7 @@ int lrbms_online_debug_timing(lrbms_plan_t plan, int64_t* out_host, int32_t n) {
   if (!plan || plan->kind != PLAN_ONLINE || !out_host) return LRBMS_ERR_INVALID;
   OnlinePlan* P = static_cast<OnlinePlan*>(plan);
 #ifdef LRBMS_DEVTOOLS
-  long long* src = P->use_v3 ? P->v3.timing : (P->use_v2 ? P->sp2.timing : nullptr);
+  long long* src = P->solver == LRBMS_SOLVER_WINDOW ? P->sp2.timing : nullptr;
   if (!src) return lrbms_fail(P->ctx, LRBMS_ERR_INVALID, "debug timing is off (set LRBMS_SOLVE_TIMING=1 before creating the plan)");
   const int cnt = std::min<int>(n, kV2Warps * 8);
   LRBMS_CUDA_CHECK(P->ctx, cudaMemcpy(out_host, src, sizeof(long long) * cnt, cudaMemcpyDeviceToHost));

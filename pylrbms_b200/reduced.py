@@ -225,7 +225,7 @@ class ReducedModel:
         self._plan_has_estimator = False
         self._work = {}
         self.linear = True
-        self.solver = 'auto'        # 'auto' | 'window' | 'banded' | 'global_tiles' (lrbms_sm100.h LRBMS_SOLVER_*)
+        self.solver = 'auto'        # 'auto' | 'window' | 'banded' (lrbms_sm100.h LRBMS_SOLVER_*)
 
     def with_(self, **kw):
         new = copy.copy(self)
@@ -341,8 +341,7 @@ class ReducedModel:
         sysc.n_sub, sysc.basis_sizes, sysc.Q, sysc.Qf = S, sizes.ctypes.data, Q, Qf
         sysc.n_blocks, sysc.block_i, sysc.block_j, sysc.block_offset = len(pattern), bi.ctypes.data, bj.ctypes.data, boff.ctypes.data
         sysc.lhs_blocks, sysc.rhs = buf.data_ptr(), rhs.data_ptr()
-        sysc.solver = {'auto': L.SOLVER_AUTO, 'window': L.SOLVER_WINDOW, 'global_tiles': L.SOLVER_GLOBAL_TILES,
-                       'banded': L.SOLVER_BANDED, 'panel': L.SOLVER_PANEL}[self.solver]
+        sysc.solver = {'auto': L.SOLVER_AUTO, 'window': L.SOLVER_WINDOW, 'banded': L.SOLVER_BANDED}[self.solver]
         keep = [bi, bj, boff, sizes, rhs, buf]
         has_est = self.estimator is not None and all('nc_{}'.format(s) in self.operators for s in self.estimator.subdomains)
         if has_est:
@@ -379,7 +378,7 @@ class ReducedModel:
         return self._plan
 
     def set_solver(self, solver):
-        """Select the solve kernel of the online plan ('auto', 'window', 'banded', 'global_tiles'); drops a built plan."""
+        """Select the solve kernel of the online plan ('auto', 'window', 'banded'); drops a built plan."""
         if solver != self.solver:
             self.solver, self._plan, self._work = solver, None, {}
         return self

@@ -31,7 +31,7 @@ def test_binding_covers_header(built_library):
     from pylrbms_b200 import _lib
     assert sorted(_lib.EXPORTS) == _declared_symbols()
     lib = _lib.load_library()
-    assert lib.lrbms_version() == 100
+    assert lib.lrbms_version() == 101
 
 
 _NO_DEVICE_CHECK = '''
@@ -77,7 +77,8 @@ def _grid_blocks(sx, sy):
 @pytest.mark.parametrize('sx,sy,sizes', [(1, 1, [5]), (2, 2, [8] * 4), (3, 2, [3, 11, 7, 20, 1, 9]), (4, 4, [20] * 16),
                                          (3, 3, [0, 4, 9, 2, 0, 17, 8, 8, 1])])
 def test_symbolic_schedule_replays_to_cholesky(built_library, sx, sy, sizes):
-    """Replay the left-looking 8x8-tile schedule of csrc/symbolic.cpp in NumPy, exactly as solve_kernel consumes it."""
+    """Replay the left-looking 8x8-tile schedule of csrc/symbolic.cpp in NumPy: its pair lists are what the window
+    schedule of solve_kernel_v2 is built from."""
     from pylrbms_b200._lib import Symbolic
     rng = np.random.default_rng(3)
     blocks = _grid_blocks(sx, sy)

@@ -296,10 +296,6 @@ def _solve(handle, plan, theta, n_red):
 
 @pytest.mark.parametrize('solver,large,small', [
     (1, (8, 8, 20, 2), (2, 2, 8, 1)),         # window kernel (v2)
-    # global-tile kernel (v1): its shared-memory vector holds the whole solution, n_red = 7 168 and 6 144 -- both plans
-    # above the 48 KB that need a raised limit, the second below the first
-    (2, (16, 16, 28, 2), (16, 16, 24, 2)),
-    (4, (8, 8, 20, 2), (2, 2, 8, 1)),         # panel kernel (v3)
 ])
 def test_large_solve_plan_runs_after_smaller_plan(handle, solver, large, small):
     """The dynamic shared-memory limit is an attribute of the kernel, shared by all plans: creating a plan with a smaller

@@ -443,18 +443,17 @@ def _run_sweep(handle, plan, sysd, theta, with_est):
     (4, 4, [20] * 16),
     (8, 8, [20] * 64),                               # C2 reduced-system shape
 ])
-@pytest.mark.parametrize('solver', [1, 2, 3, 4])
+@pytest.mark.parametrize('solver', [1, 3])
 def test_online_solve_matches_dense(handle, sx, sy, sizes, solver):
-    """All four solve kernels (lrbms_sm100.h LRBMS_SOLVER_*): 4 the two-column panel kernel (what AUTO picks when its
-    schedule applies and the window fits), 1 the one-column shared-memory window kernel, 2 the first-generation
-    global-scratch tile kernel, 3 the block-banded out-of-HBM Cholesky (what AUTO picks for large systems)."""
+    """Both solve kernels (lrbms_sm100.h LRBMS_SOLVER_*): 1 the shared-memory window kernel (what AUTO picks when the
+    window fits one SM), 3 the block-banded out-of-HBM Cholesky (what AUTO picks for large systems).  Any other solver
+    value is rejected at plan creation."""
+    from pylrbms_b200._lib import LrbmsError
     rng = np.random.default_rng(10 + sx * 7 + sy)
     sysd = _random_reduced_system(rng, sx, sy, sizes)
-    if solver == 4 and ((sysd['n'] + 7) // 8) % 2:
-        from pylrbms_b200._lib import LrbmsError
-        with pytest.raises(LrbmsError, match='panel kernel does not apply'):       # odd number of tile columns
-            _make_online_plan(handle, sysd, solver=solver)
-        return
+    for retired in (2, 4):
+        with pytest.raises(LrbmsError, match='unknown solver'):
+            _make_online_plan(handle, sysd, solver=retired)
     plan, _ = _make_online_plan(handle, sysd, solver=solver)
     out = C.c_double()
     handle.check(handle.lib.lrbms_plan_info(plan.p, 6, C.byref(out)))
@@ -535,7 +534,7 @@ def test_band_solver_large_systems(handle, shape, N, n_mu):
     assert infob[2] > 0 and np.all(infob[[0, 1, 3]] == 0) and np.array_equal(ub[[0, 1, 3]], u[[0, 1, 3]])
 
 
-@pytest.mark.parametrize('solver', [4, 1])
+@pytest.mark.parametrize('solver', [1])
 def test_online_solve_is_bit_reproducible(handle, solver):
     """The column pipeline of solve_kernel_v2 lets the two halves of its update warps run the triangular solve and the pair
     loop in opposite order with a single barrier per tile column; a data race there would show as run-to-run differences.

@@ -60,7 +60,7 @@ CASES = [
     # 3D structure of config C4 (six face neighbours), synthetic operators
     ((2, 2, 2), (2, 2, 2), [5, 6, 7, 4, 8, 6, 5, 7], 11),
     ((3, 3, 3), (2, 2, 2), 8, 12),           # the centre subdomain has a seven-member neighbourhood
-    ((3, 3, 3), (3, 3, 3), 40, 13),          # N = 40: global-scratch solve kernel, 16-parameter estimator CTAs
+    ((3, 3, 3), (3, 3, 3), 40, 13),          # N = 40: 16-parameter estimator CTAs
 ]
 
 

@@ -1,12 +1,12 @@
-"""Developer aid: in-kernel cycle counters of the shared-memory solve kernels (CTA 0, per warp and phase).
+"""Developer aid: in-kernel cycle counters of the shared-memory solve kernel (CTA 0, per warp and phase).
 
-    LRBMS_DEVTOOLS=1 python -m pylrbms_b200.build --force && python tools/solve_timing.py [--solver panel|window]
+    LRBMS_DEVTOOLS=1 python -m pylrbms_b200.build --force && python tools/solve_timing.py [--solver window|auto]
 
 Needs a library built with -DLRBMS_DEVTOOLS (never the shipped build)."""
 import os, sys, numpy as np, ctypes as C
 os.environ['LRBMS_SOLVE_TIMING'] = '1'
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-solver = 'panel'
+solver = 'window'
 if '--solver' in sys.argv:
     i = sys.argv.index('--solver'); solver = sys.argv[i + 1]; del sys.argv[i:i + 2]
 import torch, bench
@@ -26,12 +26,8 @@ out = np.zeros(128, dtype=np.int64)
 n = plan.handle.lib.lrbms_online_debug_timing(plan.p, out.ctypes.data, 128)
 assert n == 128, plan.handle.lib.lrbms_last_error(plan.handle.h)
 t = out.reshape(16, 8) / 8.0            # per parameter
-if solver == 'panel':
-    names = ['A:early', 'bar_all', 'stage|head', 'rows|diag', 'barX', 'B2|chain', 'wait+bar', 'backward']
-    div, what = 80, 'panel'
-else:
-    names = ['meta', 'chain|Y', 'ubar', 'X', 'endbar', 'epi', 'back', 'store']
-    div, what = 160, 'column'
+names = ['meta', 'chain|Y', 'ubar', 'X', 'endbar', 'epi', 'back', 'store']
+div, what = 160, 'column'
 print('kernel', rd.solve_kernel_name, ' launch of', n_mu, 'parameters: %.3f ms' % e0.elapsed_time(e1))
 print('cycles per parameter, per warp:')
 print('warp ' + ' '.join('%9s' % n for n in names) + '   total')
