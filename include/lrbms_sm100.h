@@ -200,14 +200,23 @@ int lrbms_plan_info(lrbms_plan_t plan, int32_t what, double* out);
 int lrbms_symbolic_create(int32_t n_sub, const int32_t* basis_sizes, int32_t n_blocks, const int32_t* block_i,
                           const int32_t* block_j, lrbms_symbolic_t* out);
 int lrbms_symbolic_destroy(lrbms_symbolic_t s);
+/* Elimination order (what online plans do once the shared-memory window kernel is selected): re-plan the schedule of s,
+ * built in the given subdomain order, in the cheapest of the given order, the Cuthill-McKee level-set order of the
+ * subdomain graph and its reverse, by a column-period model of the window kernel.  A candidate is only taken if it keeps
+ * the staggered schedule variant of the given order and its kernel shared memory for Q operator terms stays within
+ * smem_budget bytes; the given order wins ties.  Fails with LRBMS_ERR_INVALID if s was already re-planned. */
+int lrbms_symbolic_reorder(lrbms_symbolic_t s, int32_t Q, int64_t smem_budget);
 /* what: 0 n_red, 1 padded n, 2 tile columns, 3 L tiles, 4 A tiles, 5 update pairs, 6 factor flops per mu,
  *       7 max targets per tile column, 8 shared-memory window slots (live off-diagonal L tiles, peak),
  *       11 schedule variant of the shared-memory kernel: 1 = early updates stop at source column J - 3 and the pair with
- *          source column J - 2 rides with the late update (every such pair has a carrier tile), 0 = barrier schedule */
+ *          source column J - 2 rides with the late update (every such pair has a carrier tile), 0 = barrier schedule,
+ *       12 elimination order (0 given, 1 Cuthill-McKee, 2 reverse Cuthill-McKee), 13 / 14 / 15 modelled SM cycles per
+ *          parameter of the given / CM / RCM order (after lrbms_symbolic_reorder; 0 = not evaluated) */
 int lrbms_symbolic_info(lrbms_symbolic_t s, int32_t what, int64_t* out);
 /* copy out schedule arrays (for tests): which: 0 col_ptr[ntc+1], 1 row_idx[n_tiles], 2 pair_ptr[n_tiles+ntc+1],
  * 3 pair_a, 4 pair_b, 5 a_map[n_tiles], 6 win_slot[n_tiles], 7 late_ptr[n_tiles+ntc], 8 win_a[pairs], 9 win_b[pairs],
- * 10 xo_ptr[ntc+1], 11 xo_idx[n_tiles+ntc], 12 cnext[n_tiles+ntc], 13 chas[ntc], 14 cord[n_tiles+ntc];
+ * 10 xo_ptr[ntc+1], 11 xo_idx[n_tiles+ntc], 12 cnext[n_tiles+ntc], 13 chas[ntc], 14 cord[n_tiles+ntc],
+ * 15 perm[n_sub] (subdomain eliminated k-th), 16 iperm[n_sub], 17 row_map[n_red] (given row of every permuted row);
  * returns number of int32 written (<= cap) or a negative status */
 int64_t lrbms_symbolic_get(lrbms_symbolic_t s, int32_t which, int32_t* out, int64_t cap);
 

@@ -20,7 +20,7 @@ EXPORTS = [
     'lrbms_va_transpose_in', 'lrbms_va_transpose_out',
     'lrbms_spmm_plan_create', 'lrbms_project_plan_create', 'lrbms_project_plan_scratch_bytes',
     'lrbms_project_plan_create_ws', 'lrbms_plan_run', 'lrbms_plan_destroy', 'lrbms_plan_info',
-    'lrbms_symbolic_create', 'lrbms_symbolic_destroy', 'lrbms_symbolic_info', 'lrbms_symbolic_get',
+    'lrbms_symbolic_create', 'lrbms_symbolic_destroy', 'lrbms_symbolic_info', 'lrbms_symbolic_get', 'lrbms_symbolic_reorder',
     'lrbms_online_plan_create', 'lrbms_online_workspace_bytes', 'lrbms_online_solve', 'lrbms_online_estimate',
     'lrbms_online_sweep', 'lrbms_eta_max', 'lrbms_online_debug_timing',
     'lrbms_pcg_workspace_bytes', 'lrbms_pcg_solve', 'lrbms_remap_blocks', 'lrbms_peer_push',
@@ -116,6 +116,7 @@ def load_library():
             'lrbms_symbolic_destroy': (C.c_int, [vp]),
             'lrbms_symbolic_info': (C.c_int, [vp, i32, P(i64)]),
             'lrbms_symbolic_get': (i64, [vp, i32, vp, i64]),
+            'lrbms_symbolic_reorder': (C.c_int, [vp, i32, i64]),
             'lrbms_online_plan_create': (C.c_int, [vp, vp, P(vp)]),
             'lrbms_online_workspace_bytes': (C.c_int, [vp, i64, P(C.c_size_t)]),
             'lrbms_online_solve': (C.c_int, [vp, i64, vp, vp, vp, vp, C.c_size_t, vp]),
@@ -273,6 +274,7 @@ class Symbolic:
         if rc != 0:
             raise LrbmsError('lrbms_symbolic_create failed ({})'.format(rc))
         self.s = s
+        self.n_sub = len(sizes)
 
     def info(self, what):
         out = C.c_int64()
@@ -291,12 +293,22 @@ class Symbolic:
     max_targets = property(lambda self: self.info(7))
     n_win_slots = property(lambda self: self.info(8))
     staggered = property(lambda self: self.info(11))
+    order = property(lambda self: self.info(12))                 # 0 given, 1 Cuthill-McKee, 2 reverse Cuthill-McKee
+    order_costs = property(lambda self: tuple(self.info(k) for k in (13, 14, 15)))
+
+    def reorder(self, Q, smem_budget):
+        """Re-plan in the cheapest subdomain order that fits ``smem_budget`` bytes (see lrbms_symbolic_reorder)."""
+        rc = self.lib.lrbms_symbolic_reorder(self.s, int(Q), int(smem_budget))
+        if rc != 0:
+            raise LrbmsError('lrbms_symbolic_reorder failed ({})'.format(rc))
+        return self.order
 
     def get(self, which):
         sizes = {0: self.n_tile_cols + 1, 1: self.n_tiles, 2: self.n_tiles + self.n_tile_cols + 1, 3: self.n_pairs,
                  4: self.n_pairs, 5: self.n_tiles, 6: self.n_tiles, 7: self.n_tiles + self.n_tile_cols, 8: self.n_pairs,
                  9: self.n_pairs, 10: self.n_tile_cols + 1, 11: self.n_tiles + self.n_tile_cols,
-                 12: self.n_tiles + self.n_tile_cols, 13: self.n_tile_cols, 14: self.n_tiles + self.n_tile_cols}
+                 12: self.n_tiles + self.n_tile_cols, 13: self.n_tile_cols, 14: self.n_tiles + self.n_tile_cols,
+                 15: self.n_sub, 16: self.n_sub, 17: self.n_red}
         out = np.zeros(sizes[which], dtype=np.int32)
         n = self.lib.lrbms_symbolic_get(self.s, which, ptr(out), out.size)
         if n != out.size:

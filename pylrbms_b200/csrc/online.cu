@@ -7,7 +7,9 @@
 // A_IJ(mu) - sum_K L_IK L_JK^T is accumulated with DMMA (A_IJ(mu) = sum_q theta_q(mu) A_q is assembled on the fly, left
 // to right like LincombOperator.assemble), the diagonal tile is factored and inverted, and the off-diagonal tiles are
 // multiplied by L_JJ^{-T}.  The right-hand side rides along as one more tile row (forward substitution fused into the
-// factorisation).  Systems whose window does not fit one SM's shared memory go to the band solver (band.cu).
+// factorisation).  Systems whose window does not fit one SM's shared memory go to the band solver (band.cu).  The kernel
+// factors P A P^T with the subdomains in the elimination order the symbolic phase chose (lrbms_symbolic_choose_order);
+// the operator tiles and the rhs are uploaded permuted, u and the failed-pivot row go back through a row map.
 //
 // estimate_kernel: one CTA per (subdomain, tile of 32 parameters).  Every quadratic form x_L^T M x_R of
 // reference estimators.py:71-85 is evaluated for 32 parameters at once as Y = M X_R on DMMA followed by a column dot
@@ -32,15 +34,13 @@ namespace {
 //    * targets of a column are handed out dynamically (longest first) through a shared-memory counter;
 //    * the backward substitution streams the factor back with a 4-stage cp.async ring.
 // ------------------------------------------------------------------------------------------------------
-constexpr int kV2Threads = 512;
-constexpr int kV2Warps = kV2Threads / 32;
-constexpr int kBackStages = 6;     // backward-substitution ring; columns are prefetched kBackStages - 2 ahead
-constexpr int kMetaBufs = 5;     // column metadata: columns J-1 .. J+3 are alive at the same time (staged by cp.async)
-constexpr int kABufs = 3;        // staged operator tiles: only needed while a column's early updates run
+// (kV2Warps, kBackStages, kMetaBufs and kABufs are in symbolic.h: the symbolic phase sizes the shared memory with them)
+constexpr int kV2Threads = kV2Warps * 32;
 
 struct SolveParamsV2 {
   int32_t n_red, n_pad, Q, Qf, n_theta, n_a_tiles, ntc;
   const int32_t* row_idx;   // [n_tiles] tile row of every factor slot
+  const int32_t* row_map;   // [n_red] row of u (the caller's order) of every row of the permuted system
   const double* a_tiles;    // [Q][n_a_tiles][64]
   const double* rhs;        // [Qf][n_pad]
   int64_t work_stride;      // doubles of factor scratch per CTA: n_tiles * 64
@@ -57,7 +57,7 @@ struct SolveParamsV2 {
   int32_t region_doubles;   // shared-memory window region (also the backward-substitution ring)
   int32_t max_targets;      // per column, incl. the diagonal tile and the rhs row
   int32_t max_col_pairs;
-  int32_t max_a_col;
+  int32_t a_ring;           // operator-tile slots of the staging ring (lrbms_symbolic::a_ring)
   int32_t back_stage_doubles;
   int32_t staggered;        // schedule variant of the symbolic phase (lrbms_symbolic::staggered)
 #ifdef LRBMS_DEVTOOLS
@@ -110,9 +110,9 @@ solve_kernel_v2(SolveParamsV2 P, int64_t n_mu, const double* __restrict__ theta,
   double* sScr = sW + 2 * 64;                                 // 2 * 64: layout-conversion scratch (shared tile, chain warp)
   double* sred = sScr + 2 * 64;                               // 2 * kV2Warps * 8
   double* sth = sred + 2 * kV2Warps * 8;                      // n_theta (<= 32)
-  double* sA = sth + 32;                                      // kABufs * max_a_col * Q * 64
-  const int a_buf_doubles = P.max_a_col * P.Q * 64;
-  int4* sDesc = reinterpret_cast<int4*>(sA + kABufs * a_buf_doubles);             // kMetaBufs * MT
+  double* sA = sth + 32;                                      // a_ring * Q * 64
+  const int a_tile_doubles = P.Q * 64;
+  int4* sDesc = reinterpret_cast<int4*>(sA + P.a_ring * a_tile_doubles);          // kMetaBufs * MT
   int4* sCol = sDesc + kMetaBufs * MT;                                            // ntc + 1
   int4* sCol2 = sCol + (P.ntc + 1);                                               // ntc
   int4* sCol3 = sCol2 + P.ntc;                                                    // ntc
@@ -143,7 +143,7 @@ solve_kernel_v2(SolveParamsV2 P, int64_t n_mu, const double* __restrict__ theta,
   for (int i = threadIdx.x; i < P.n_ca; i += kV2Threads) sCaTile[i] = P.ca_tile[i];
   __syncthreads();
 
-  // stage everything column Jn needs into buffer Jn % kMetaBufs / Jn % kABufs.  Called by ONE producer warp (the
+  // stage everything column Jn needs into buffer Jn % kMetaBufs and the operator-tile ring.  Called by ONE producer warp (the
   // address arithmetic is a long dependent chain; keeping it off the other 15 warps takes it off the critical path);
   // asynchronous copies, one commit group per call
   auto stage_meta = [&](int Jn) {
@@ -162,12 +162,14 @@ solve_kernel_v2(SolveParamsV2 P, int64_t n_mu, const double* __restrict__ theta,
       for (int i = lane; i < ci.y; i += 32) cp_async8(dst + i, P.win_ab + ci.x + i);
       for (int i = lane; i < ci.w; i += 32) cp_async8(dst + ci.y + i, P.win_ab + ci.z + i);
       // raw operator tiles A_q of the column's targets (the theta-weighted sum is formed when they are consumed):
-      // one 16-byte chunk per lane, 32 lanes = one tile per step
-      double* adst = sA + (Jn % kABufs) * a_buf_doubles;
+      // one 16-byte chunk per lane, 32 lanes = one tile per step.  Tile k of the column goes to ring slot
+      // (c3.x + k) mod a_ring: the tiles of the kABufs columns alive at a time never share a slot.
+      int slot = c3.x % P.a_ring;
       for (int k = 0; k < c3.y; ++k) {
         const int64_t src_tile = sCaTile[c3.x + k];
         for (int q = 0; q < P.Q; ++q)
-          cp_async16(adst + (k * P.Q + q) * 64 + lane * 2, P.a_tiles + ((int64_t)q * P.n_a_tiles + src_tile) * 64 + lane * 2);
+          cp_async16(sA + (slot * P.Q + q) * 64 + lane * 2, P.a_tiles + ((int64_t)q * P.n_a_tiles + src_tile) * 64 + lane * 2);
+        if (++slot == P.a_ring) slot = 0;
       }
     }
     cp_async_commit();
@@ -183,7 +185,7 @@ solve_kernel_v2(SolveParamsV2 P, int64_t n_mu, const double* __restrict__ theta,
     const int4* descC = sDesc + mb * MT;
     const int2* pairC = sPair + mb * P.max_col_pairs;
     const int* ordC = sOrd + mb * MT;
-    const double* aC = sA + (Jx % kABufs) * a_buf_doubles;
+    const int a_first = sCol3[Jx].x % P.a_ring;               // ring slot of the column's first staged operator tile
     const int ncol = sCol[Jx].y;
     // Snake deal over the 14 update warps (1..14), longest item first.  (The triangular solve gives warps
     // 1 .. n_tiles - 14 two tiles and the others one, so the longest early items go to the *high* warps: warp 14 first.)
@@ -207,7 +209,8 @@ solve_kernel_v2(SolveParamsV2 P, int64_t n_mu, const double* __restrict__ theta,
       double a0 = 0.0, a1 = 0.0;
       if (li < ncol) {
         if (d.w >= 0) {                                        // A(mu) tile = sum_q theta_q A_q, left to right
-          const double* at = aC + d.w * P.Q * 64 + g * 8 + 2 * t;
+          const int slot = (a_first + d.w < P.a_ring) ? a_first + d.w : a_first + d.w - P.a_ring;
+          const double* at = sA + slot * a_tile_doubles + g * 8 + 2 * t;
           for (int q = 0; q < P.Q; ++q) {
             const double2 v = *reinterpret_cast<const double2*>(at + q * 64);
             if (q == 0) { a0 = sth[0] * v.x; a1 = sth[0] * v.y; }
@@ -553,8 +556,9 @@ solve_kernel_v2(SolveParamsV2 P, int64_t n_mu, const double* __restrict__ theta,
       cp_async_wait<0>();
     }
     LRBMS_TICK(6);
-    for (int i = threadIdx.x; i < P.n_red; i += kV2Threads) u[mu * P.n_red + i] = sx[i];
-    if (threadIdx.x == 0 && info) info[mu] = s_info;
+    // back to the caller's row order; a failed pivot is reported as its row there
+    for (int i = threadIdx.x; i < P.n_red; i += kV2Threads) u[mu * P.n_red + __ldg(P.row_map + i)] = sx[i];
+    if (threadIdx.x == 0 && info) info[mu] = s_info ? __ldg(P.row_map + s_info - 1) + 1 : 0;
     LRBMS_TICK(7);
   }
 #ifdef LRBMS_DEVTOOLS
@@ -822,7 +826,7 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
   const lrbms_symbolic& S = P->sym;
   const int Q = sys->Q, Qf = sys->Qf;
 
-  // ---- operator tiles: download the reduced blocks, scatter the lower triangle into 8x8 tiles
+  // ---- download the reduced blocks and the rhs
   int64_t n_doubles = 0;
   for (int q = 0; q < Q; ++q)
     for (int b = 0; b < sys->n_blocks; ++b)
@@ -833,37 +837,10 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
     cudaError_t e = cudaMemcpy(hb.data(), sys->lhs_blocks, sizeof(double) * n_doubles, cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) { delete P; return lrbms_fail(h, LRBMS_ERR_CUDA, cudaGetErrorString(e)); }
   }
-  std::vector<double> tiles;
-  if (tiles_built) {
-  tiles.assign((size_t)Q * S.n_a_tiles * 64, 0.0);
-  auto slot_of = [&](int I, int J) {
-    const int32_t* b = S.row_idx.data() + S.col_ptr[J];
-    const int32_t* e = S.row_idx.data() + S.col_ptr[J + 1];
-    return (int32_t)(std::lower_bound(b, e, I) - S.row_idx.data());
-  };
-  for (int q = 0; q < Q; ++q)
-    for (int b = 0; b < sys->n_blocks; ++b) {
-      const int i = sys->block_i[b], j = sys->block_j[b];
-      if (i < j) continue;
-      const double* blk = hb.data() + sys->block_offset[(int64_t)q * sys->n_blocks + b];
-      const int Ni = S.sizes[i], Nj = S.sizes[j];
-      for (int a = 0; a < Ni; ++a)
-        for (int c = 0; c < Nj; ++c) {
-          const int r = S.offsets[i] + a, cc = S.offsets[j] + c;
-          if (r < cc) continue;
-          const int ai = S.a_map[slot_of(r / 8, cc / 8)];
-          double* tl = tiles.data() + ((size_t)q * S.n_a_tiles + ai) * 64;
-          tl[(r & 7) * 8 + (cc & 7)] = blk[(int64_t)a * Nj + c];
-          if (r / 8 == cc / 8) tl[(cc & 7) * 8 + (r & 7)] = blk[(int64_t)a * Nj + c];
-        }
-    }
-  }
-  std::vector<double> rhs_h((size_t)Qf * S.n_pad, 0.0);
   std::vector<double> tmp((size_t)Qf * S.n_red);     // [Qf][n_red], as given
   {
     cudaError_t e = cudaMemcpy(tmp.data(), sys->rhs, sizeof(double) * tmp.size(), cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) { delete P; return lrbms_fail(h, LRBMS_ERR_CUDA, cudaGetErrorString(e)); }
-    for (int q = 0; q < Qf; ++q) std::copy(tmp.begin() + (size_t)q * S.n_red, tmp.begin() + (size_t)(q + 1) * S.n_red, rhs_h.begin() + (size_t)q * S.n_pad);
   }
 
 // CUDA calls after the plan object exists: destroy it on failure (no leaked plans on error paths)
@@ -881,29 +858,59 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
 #define UP_F64(field, vec) do { rc = plan_upload(P, &d_f64, vec); if (rc) { lrbms_plan_destroy(P); return rc; } field = d_f64; } while (0)
   // ---- shared-memory-window kernel: used whenever the live window of L fits into the shared memory of one SM
   if (tiles_built) {
-    const int maxcol = std::max(1, S.max_targets - 1);
-    const int MT = S.max_targets;
-    const int64_t region = std::max<int64_t>((int64_t)S.n_win_slots * 64, (int64_t)kBackStages * maxcol * 64);
-    const int mcp = std::max(1, S.max_col_pairs), mac = std::max(1, S.max_a_col);
-    const size_t bytes = sizeof(double) * ((size_t)region + 3 * (size_t)MT * 64 + S.n_pad + 4 * 64 + 2 * kV2Warps * 8 + 32 +
-                                           (size_t)kABufs * mac * Q * 64) +
-                         16 * ((size_t)kMetaBufs * MT + (size_t)(S.ntc + 1) + 2 * (size_t)S.ntc) + 8 * (size_t)kMetaBufs * mcp +
-                         4 * (3 * (size_t)kMetaBufs * MT + S.ca_tile.size()) + 64;
     size_t static2 = 0;
     PLAN_CUDA_CHECK(lrbms_open_dynamic_smem(h, (const void*)solve_kernel_v2, &static2));
     // the static shared memory of the kernel (mbarriers, status word) counts against the same per-block limit
-    if (bytes + static2 <= (size_t)h->max_smem_optin) {
+    const int64_t smem_budget = (int64_t)h->max_smem_optin - (int64_t)static2;
+    if ((int64_t)lrbms_window_smem_bytes(S, Q) <= smem_budget) {
+      // The window kernel runs; factor in the subdomain order its cost model prefers (within the same shared memory).
+      rc = lrbms_symbolic_choose_order(P->sym, Q, smem_budget, &err);
+      if (rc) { lrbms_plan_destroy(P); return lrbms_fail(h, rc, err); }
+      const int maxcol = std::max(1, S.max_targets - 1);
+      const int MT = S.max_targets;
+      const int64_t region = std::max<int64_t>((int64_t)S.n_win_slots * 64, (int64_t)kBackStages * maxcol * 64);
+      const int mcp = std::max(1, S.max_col_pairs);
+      // operator tiles of the permuted system: the lower triangle of every stored block (i >= j) goes to its permuted
+      // rows and columns, transposed where the order puts subdomain j after subdomain i
+      std::vector<double> tiles((size_t)Q * S.n_a_tiles * 64, 0.0);
+      auto slot_of = [&](int I, int J) {
+        const int32_t* b = S.row_idx.data() + S.col_ptr[J];
+        const int32_t* e = S.row_idx.data() + S.col_ptr[J + 1];
+        return (int32_t)(std::lower_bound(b, e, I) - S.row_idx.data());
+      };
+      for (int q = 0; q < Q; ++q)
+        for (int b = 0; b < sys->n_blocks; ++b) {
+          const int i = sys->block_i[b], j = sys->block_j[b];
+          if (i < j) continue;
+          const double* blk = hb.data() + sys->block_offset[(int64_t)q * sys->n_blocks + b];
+          const int Ni = S.sizes[i], Nj = S.sizes[j];
+          const bool flip = S.iperm[i] < S.iperm[j];
+          for (int a = 0; a < Ni; ++a)
+            for (int c = 0; c < Nj; ++c) {
+              int r = S.perm_offsets[i] + a, cc = S.perm_offsets[j] + c;
+              if (flip) std::swap(r, cc);
+              if (r < cc) continue;
+              const int ai = S.a_map[slot_of(r / 8, cc / 8)];
+              double* tl = tiles.data() + ((size_t)q * S.n_a_tiles + ai) * 64;
+              tl[(r & 7) * 8 + (cc & 7)] = blk[(int64_t)a * Nj + c];
+              if (r / 8 == cc / 8) tl[(cc & 7) * 8 + (r & 7)] = blk[(int64_t)a * Nj + c];
+            }
+        }
+      std::vector<double> rhs_h((size_t)Qf * S.n_pad, 0.0);
+      for (int q = 0; q < Qf; ++q)
+        for (int r = 0; r < S.n_red; ++r) rhs_h[(size_t)q * S.n_pad + r] = tmp[(size_t)q * S.n_red + S.row_map[r]];
       SolveParamsV2& s2 = P->sp2;
       s2.n_red = S.n_red; s2.n_pad = S.n_pad; s2.ntc = S.ntc; s2.Q = Q; s2.Qf = Qf; s2.n_theta = Q + Qf;
       s2.n_a_tiles = S.n_a_tiles;
       s2.work_stride = (int64_t)S.n_tiles() * 64;
       UP_I32(s2.row_idx, S.row_idx);
+      UP_I32(s2.row_map, S.row_map);
       UP_F64(s2.a_tiles, tiles);
       UP_F64(s2.rhs, rhs_h);
       s2.region_doubles = (int32_t)region;
       s2.max_targets = MT;
       s2.max_col_pairs = mcp;
-      s2.max_a_col = mac;
+      s2.a_ring = S.a_ring;
       s2.back_stage_doubles = maxcol * 64;
       s2.n_ca = (int32_t)S.ca_tile.size();
       UP_I32(s2.cslot, S.cslot);
@@ -927,7 +934,7 @@ int lrbms_online_plan_create(lrbms_handle_t h, const lrbms_reduced_system_t* sys
         }
       }
 #endif
-      P->solve_smem = bytes;
+      P->solve_smem = lrbms_window_smem_bytes(S, Q);
       P->solver = LRBMS_SOLVER_WINDOW;
       P->solve_grid = h->sm_count;
       P->solve_stride = s2.work_stride;

@@ -274,6 +274,14 @@ int lrbms_symbolic_build(lrbms_symbolic& S, int32_t n_sub, const int32_t* sizes,
       S.ccol3[4 * J + 1] = na;
       S.max_a_col = std::max(S.max_a_col, na);
     }
+    // the staged tiles of kABufs consecutive columns are alive at the same time; they sit in a ring of operator-tile slots
+    // (tile k of column J in slot (ccol3[J].x + k) mod a_ring)
+    S.a_ring = 1;
+    for (int J = 0; J < S.ntc; ++J) {
+      int32_t live = 0;
+      for (int d = 0; d < kABufs && J + d < S.ntc; ++d) live += S.ccol3[4 * (J + d) + 1];
+      S.a_ring = std::max(S.a_ring, live);
+    }
     // consumers of the "late" update: tile (I, J) feeds target (I, J + 1) together with tile (J + 1, J)
     S.cnext.assign(n_items_total, -1);
     S.chas.assign(S.ntc, 0);
@@ -303,6 +311,174 @@ int lrbms_symbolic_build(lrbms_symbolic& S, int32_t n_sub, const int32_t* sizes,
   S.flops = 0;
   for (int64_t tgt = 0; tgt < n_tiles; ++tgt) S.flops += (int64_t)count[tgt] * 1024;
   S.flops += n_tiles * 1024;
+  // given order
+  S.order = LRBMS_ORDER_GIVEN;
+  S.perm.resize(n_sub);
+  for (int i = 0; i < n_sub; ++i) S.perm[i] = i;
+  S.iperm = S.perm;
+  S.perm_offsets.assign(S.offsets.begin(), S.offsets.end() - 1);
+  S.row_map.resize(S.n_red);
+  for (int r = 0; r < S.n_red; ++r) S.row_map[r] = r;
+  return LRBMS_OK;
+}
+
+size_t lrbms_window_smem_bytes(const lrbms_symbolic& S, int Q) {
+  const int maxcol = std::max(1, S.max_targets - 1);
+  const size_t MT = (size_t)S.max_targets;
+  const size_t region = (size_t)std::max<int64_t>((int64_t)S.n_win_slots * 64, (int64_t)kBackStages * maxcol * 64);
+  const size_t mcp = (size_t)std::max(1, S.max_col_pairs);
+  return sizeof(double) * (region + 3 * MT * 64 + S.n_pad + 4 * 64 + 2 * kV2Warps * 8 + 32 + (size_t)S.a_ring * Q * 64) +
+         16 * ((size_t)kMetaBufs * MT + (size_t)(S.ntc + 1) + 2 * (size_t)S.ntc) + 8 * (size_t)kMetaBufs * mcp +
+         4 * (3 * (size_t)kMetaBufs * MT + S.ca_tile.size()) + 64;
+}
+
+namespace {
+
+// Cuthill-McKee level-set order of the subdomain graph: per connected component (taken in order of their lowest subdomain)
+// a breadth-first search from a pseudo-peripheral subdomain; the unvisited neighbours of each subdomain are appended by
+// increasing degree (then index), so within a level subdomains follow their parent's position, then their degree.  On a
+// grid of subdomains started in a corner the levels are the anti-diagonals.
+std::vector<int32_t> cuthill_mckee(int n, const std::vector<std::vector<int32_t>>& adj) {
+  std::vector<int32_t> order, dist(n, -1);
+  order.reserve(n);
+  std::vector<char> placed(n, 0);
+  auto deg = [&](int v) { return (int)adj[v].size(); };
+  // breadth-first levels from r over r's component; returns the eccentricity of r, dist holds the levels
+  std::vector<int32_t> touched;
+  auto bfs = [&](int r) {
+    for (int v : touched) dist[v] = -1;
+    touched.assign(1, r);
+    dist[r] = 0;
+    int ecc = 0;
+    for (size_t h = 0; h < touched.size(); ++h) {
+      const int v = touched[h];
+      ecc = std::max(ecc, dist[v]);
+      for (int w : adj[v])
+        if (dist[w] < 0) { dist[w] = dist[v] + 1; touched.push_back(w); }
+    }
+    return ecc;
+  };
+  for (int s = 0; s < n; ++s) {
+    if (placed[s]) continue;
+    // pseudo-peripheral start (George and Liu): move to the lowest-degree subdomain of the last level while that
+    // increases the eccentricity
+    int root = s, ecc = bfs(s);
+    for (;;) {
+      int cand = -1;
+      for (int v : touched)
+        if (dist[v] == ecc && (cand < 0 || deg(v) < deg(cand) || (deg(v) == deg(cand) && v < cand))) cand = v;
+      const int e2 = bfs(cand);
+      if (e2 <= ecc) break;
+      root = cand;
+      ecc = e2;
+    }
+    const size_t head0 = order.size();
+    order.push_back(root);
+    placed[root] = 1;
+    for (size_t h = head0; h < order.size(); ++h) {
+      std::vector<int32_t> next;
+      for (int w : adj[order[h]])
+        if (!placed[w]) { placed[w] = 1; next.push_back(w); }
+      std::sort(next.begin(), next.end(), [&](int a, int b) { return deg(a) != deg(b) ? deg(a) < deg(b) : a < b; });
+      order.insert(order.end(), next.begin(), next.end());
+    }
+  }
+  return order;
+}
+
+// Column-period model of solve_kernel_v2 in SM cycles per parameter, fitted to the per-warp cycle counters of the C2 system
+// (8 x 8 subdomains, N = 20, lexicographic order; profiles/r02_timing_solve_v2.txt): a tile column takes at least the
+// critical chain of warp 0 (8 x 8 potrf + inverse and the hand-off to the update warps), else the update warps' work --
+// one round of triangular solves per 2 x 14 targets plus the column's update pairs spread over 14 warps, or the longest
+// single target if that is longer; the backward substitution streams every L tile once.
+double window_cost(const lrbms_symbolic& S) {
+  constexpr double kChain = 5000.0, kSolveRound = 1600.0, kPair = 300.0, kBackTile = 60.0;
+  constexpr int kUpdWarps = kV2Warps - 2;
+  const int64_t n_tiles = S.n_tiles();
+  double cost = kBackTile * (double)n_tiles;
+  for (int J = 0; J < S.ntc; ++J) {
+    const int ncol = S.col_ptr[J + 1] - S.col_ptr[J];
+    int64_t pairs = 0, longest = 0;
+    for (int32_t p = S.col_ptr[J]; p <= S.col_ptr[J + 1]; ++p) {
+      const int64_t tgt = (p < S.col_ptr[J + 1]) ? p : n_tiles + J;
+      const int64_t np = S.pair_ptr[tgt + 1] - S.pair_ptr[tgt];
+      pairs += np;
+      longest = std::max(longest, np);
+    }
+    const double rounds = (double)((ncol + 2 * kUpdWarps) / (2 * kUpdWarps));
+    const double upd = kSolveRound * rounds + kPair * std::max((double)((pairs + kUpdWarps - 1) / kUpdWarps), (double)longest);
+    cost += std::max(kChain, upd);
+  }
+  return cost;
+}
+
+}  // namespace
+
+int lrbms_symbolic_choose_order(lrbms_symbolic& S, int Q, int64_t smem_budget, std::string* err) {
+  auto fail = [&](const char* m) { if (err) *err = m; return (int)LRBMS_ERR_INVALID; };
+  if (S.order != LRBMS_ORDER_GIVEN || S.ntc == 0 || (int)S.perm.size() != S.n_sub)
+    return fail("symbolic_reorder: needs a schedule built in the given order");
+  const int n = S.n_sub;
+  std::vector<std::vector<int32_t>> adj(n);
+  for (size_t b = 0; b < S.block_i.size(); ++b) {
+    const int i = S.block_i[b], j = S.block_j[b];
+    if (i == j) continue;
+    adj[i].push_back(j);
+    adj[j].push_back(i);
+  }
+  for (auto& a : adj) {
+    std::sort(a.begin(), a.end());
+    a.erase(std::unique(a.begin(), a.end()), a.end());
+  }
+  std::vector<int32_t> cand[3];
+  cand[LRBMS_ORDER_GIVEN] = S.perm;
+  cand[LRBMS_ORDER_CM] = cuthill_mckee(n, adj);
+  cand[LRBMS_ORDER_RCM].assign(cand[LRBMS_ORDER_CM].rbegin(), cand[LRBMS_ORDER_CM].rend());
+  S.order_cost[LRBMS_ORDER_GIVEN] = window_cost(S);
+  int best = LRBMS_ORDER_GIVEN;
+  double best_cost = S.order_cost[LRBMS_ORDER_GIVEN];
+  lrbms_symbolic best_T;
+  for (int k = LRBMS_ORDER_CM; k <= LRBMS_ORDER_RCM; ++k) {
+    S.order_cost[k] = 0.0;
+    if (cand[k] == cand[LRBMS_ORDER_GIVEN]) continue;
+    // the permuted pattern: subdomain perm[k] in position k; every stored block (i >= j) lands in the lower triangle
+    std::vector<int32_t> ip(n), sizes_p(n), bi_p, bj_p;
+    for (int p = 0; p < n; ++p) { ip[cand[k][p]] = p; sizes_p[p] = S.sizes[cand[k][p]]; }
+    for (size_t b = 0; b < S.block_i.size(); ++b) {
+      const int i = S.block_i[b], j = S.block_j[b];
+      if (i < j) continue;
+      bi_p.push_back(std::max(ip[i], ip[j]));
+      bj_p.push_back(std::min(ip[i], ip[j]));
+    }
+    lrbms_symbolic T;
+    if (int rc = lrbms_symbolic_build(T, n, sizes_p.data(), (int32_t)bi_p.size(), bi_p.data(), bj_p.data(), err)) return rc;
+    S.order_cost[k] = window_cost(T);
+    if (T.staggered < S.staggered || (int64_t)lrbms_window_smem_bytes(T, Q) > smem_budget) continue;
+    if (S.order_cost[k] < best_cost) {
+      best = k;
+      best_cost = S.order_cost[k];
+      T.perm = cand[k];
+      T.iperm = ip;
+      best_T = std::move(T);
+    }
+  }
+  if (best == LRBMS_ORDER_GIVEN) return LRBMS_OK;
+  // keep the given-order description of the system (estimator, band solver, the caller's layout), take the schedule
+  lrbms_symbolic& T = best_T;
+  T.order = best;
+  for (int k = 0; k < 3; ++k) T.order_cost[k] = S.order_cost[k];
+  T.perm_offsets.resize(n);
+  T.row_map.resize(S.n_red);
+  for (int i = 0; i < n; ++i) {
+    T.perm_offsets[i] = T.offsets[T.iperm[i]];
+    for (int a = 0; a < S.sizes[i]; ++a) T.row_map[T.perm_offsets[i] + a] = S.offsets[i] + a;
+  }
+  T.sizes = std::move(S.sizes);
+  T.offsets = std::move(S.offsets);
+  T.block_i = std::move(S.block_i);
+  T.block_j = std::move(S.block_j);
+  T.half_bandwidth = S.half_bandwidth;
+  S = std::move(T);
   return LRBMS_OK;
 }
 
@@ -318,6 +494,11 @@ int lrbms_symbolic_create(int32_t n_sub, const int32_t* basis_sizes, int32_t n_b
   if (rc) { delete S; return rc; }
   *out = S;
   return LRBMS_OK;
+}
+
+int lrbms_symbolic_reorder(lrbms_symbolic_t s, int32_t Q, int64_t smem_budget) {
+  if (!s || Q < 1) return LRBMS_ERR_INVALID;
+  return lrbms_symbolic_choose_order(*s, Q, smem_budget, nullptr);
 }
 
 int lrbms_symbolic_destroy(lrbms_symbolic_t s) {
@@ -340,6 +521,8 @@ int lrbms_symbolic_info(lrbms_symbolic_t s, int32_t what, int64_t* out) {
     case 9: *out = s->max_col_pairs; break;
     case 10: *out = s->max_a_col; break;
     case 11: *out = s->staggered; break;
+    case 12: *out = s->order; break;
+    case 13: case 14: case 15: *out = (int64_t)s->order_cost[what - 13]; break;
     default: return LRBMS_ERR_INVALID;
   }
   return LRBMS_OK;
@@ -364,6 +547,9 @@ int64_t lrbms_symbolic_get(lrbms_symbolic_t s, int32_t which, int32_t* out, int6
     case 12: v = &s->cnext; break;
     case 13: v = &s->chas; break;
     case 14: v = &s->cord; break;
+    case 15: v = &s->perm; break;
+    case 16: v = &s->iperm; break;
+    case 17: v = &s->row_map; break;
     default: return LRBMS_ERR_INVALID;
   }
   const int64_t n = std::min<int64_t>(cap, (int64_t)v->size());

@@ -1,12 +1,28 @@
 // Host-only symbolic phase of the mu-batched reduced solve: 8x8-tile sparse Cholesky schedule.
 #pragma once
+#include <cstddef>
 #include <cstdint>
 #include <string>
 #include <vector>
 
+// Shape of solve_kernel_v2 (online.cu) that its shared-memory footprint depends on
+constexpr int kV2Warps = 16;
+constexpr int kBackStages = 6;   // backward-substitution ring; columns are prefetched kBackStages - 2 ahead
+constexpr int kMetaBufs = 5;     // column metadata: columns J-1 .. J+3 are alive at the same time (staged by cp.async)
+constexpr int kABufs = 3;        // staged operator tiles: only needed while a column's early updates run
+
+// Elimination order of the subdomains (lrbms_symbolic::order)
+enum { LRBMS_ORDER_GIVEN = 0, LRBMS_ORDER_CM = 1, LRBMS_ORDER_RCM = 2 };
+
 struct lrbms_symbolic {
   int32_t n_sub = 0;
-  std::vector<int32_t> sizes, offsets;   // N_i, prefix sums (n_sub + 1)
+  std::vector<int32_t> sizes, offsets;   // N_i, prefix sums (n_sub + 1), in the given subdomain order
+  // Elimination order.  The tile schedule below is that of the symmetrically permuted operator P A P^T in which
+  // subdomain perm[k] comes k-th; iperm[i] is the position of subdomain i.  perm_offsets[i] = first row of subdomain i in
+  // the permuted scalar numbering, row_map[r] = given row of permuted row r (n_red entries).  Given order: identities.
+  int32_t order = LRBMS_ORDER_GIVEN;
+  std::vector<int32_t> perm, iperm, perm_offsets, row_map;
+  double order_cost[3] = {0.0, 0.0, 0.0};   // window-kernel cost model of the given, CM and RCM order (0: not evaluated)
   int32_t n_red = 0;                     // sum N_i
   int32_t n_pad = 0;                     // n_red rounded up to a multiple of 8
   int32_t ntc = 0;                       // tile columns
@@ -52,6 +68,7 @@ struct lrbms_symbolic {
   // indices (a_map values) in staging order; cdesc[.].w is the staged position of the item's operator tile or -1
   std::vector<int32_t> ccol, ccol3, ca_tile;
   int32_t max_a_col = 0;
+  int32_t a_ring = 1;          // operator-tile slots of the staging ring: most staged tiles of kABufs consecutive columns
   int32_t max_col_pairs = 0;
 
   int64_t n_tiles() const { return (int64_t)row_idx.size(); }
@@ -63,3 +80,9 @@ int lrbms_symbolic_basics(lrbms_symbolic& S, int32_t n_sub, const int32_t* sizes
                           const int32_t* bj, std::string* err);
 int lrbms_symbolic_build(lrbms_symbolic& S, int32_t n_sub, const int32_t* sizes, int32_t n_blocks, const int32_t* bi,
                          const int32_t* bj, std::string* err);
+// dynamic shared memory (bytes) solve_kernel_v2 needs for the schedule S and Q affine operator terms
+size_t lrbms_window_smem_bytes(const lrbms_symbolic& S, int Q);
+// Re-plan S (built by lrbms_symbolic_build in the given order) in the cheapest of the given, Cuthill-McKee and reverse
+// Cuthill-McKee subdomain orders by the window kernel's cost model.  A candidate must keep the staggered schedule if the
+// given order has it and its footprint for Q terms must stay within smem_budget bytes; the given order wins ties.
+int lrbms_symbolic_choose_order(lrbms_symbolic& S, int Q, int64_t smem_budget, std::string* err);
