@@ -301,6 +301,25 @@ int lrbms_pcg_solve(lrbms_handle_t h, int32_t n, const int32_t* rowptr, const in
                     const double* b, double* x, double rtol, int32_t max_iter, int32_t* iters_out, double* relres_out,
                     void* workspace, size_t workspace_bytes, void* stream);
 
+/* Fine-scale solve of an affine operator for a batch of parameters (replaces d.solve(mu): LincombOperator.assemble(mu)
+ * + apply_inverse, dune-istl in the reference).  A(mu) = sum_q theta[mu][q] A_q on ONE CSR pattern (values: [Q][nnz],
+ * 1 <= Q <= 4, else LRBMS_ERR_UNSUPPORTED), b(mu) = sum_f theta[mu][Q + f] rhs[f] (rhs: [Qf][n]).  theta: device,
+ * row-major n_mu x (Q + Qf) -- the layout of the online plans.  x: device, dof-major n x ldx, column k = parameter k;
+ * initial guess on entry, solution on exit.  Jacobi-preconditioned CG, 32 parameters per warp-row; a parameter's result
+ * is bit-identical whatever the batch it is solved in (size, position, chunking).  A parameter whose recurrence residual
+ * reaches rtol restarts from its iterate with the true residual b - A x, at most max_restarts times and only while each
+ * restart halves the true residual; then it is frozen (its columns are no longer written).
+ * Per parameter (host arrays [n_mu]): iterations, TRUE relative residual ||b - A x|| / ||b||, status
+ * 0 = converged (true residual <= rtol), 1 = not converged within max_iter / restarts, 2 = p^T A p <= 0 met.
+ * Runs as a cooperative launch only (one CTA of 1024 threads per SM); a device that cannot gets LRBMS_ERR_UNSUPPORTED.
+ * lrbms_affine_pcg_workspace_bytes: device workspace for n_mu parameters (about 6 n doubles each); split larger batches. */
+int lrbms_affine_pcg_workspace_bytes(lrbms_handle_t h, int64_t n, int64_t n_mu, size_t* bytes);
+int lrbms_affine_pcg_solve(lrbms_handle_t h, int32_t n, int32_t Q, const int32_t* rowptr, const int32_t* colind,
+                           const double* values, int32_t Qf, const double* rhs, int64_t n_mu, const double* theta,
+                           double* x, int32_t ldx, double rtol, int32_t max_iter, int32_t max_restarts,
+                           int32_t* iters_out, double* relres_out, int32_t* status_out,
+                           void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

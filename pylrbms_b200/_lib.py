@@ -23,7 +23,8 @@ EXPORTS = [
     'lrbms_symbolic_create', 'lrbms_symbolic_destroy', 'lrbms_symbolic_info', 'lrbms_symbolic_get', 'lrbms_symbolic_reorder',
     'lrbms_online_plan_create', 'lrbms_online_workspace_bytes', 'lrbms_online_solve', 'lrbms_online_estimate',
     'lrbms_online_sweep', 'lrbms_eta_max', 'lrbms_online_debug_timing',
-    'lrbms_pcg_workspace_bytes', 'lrbms_pcg_solve', 'lrbms_remap_blocks', 'lrbms_peer_push',
+    'lrbms_pcg_workspace_bytes', 'lrbms_pcg_solve', 'lrbms_affine_pcg_workspace_bytes', 'lrbms_affine_pcg_solve',
+    'lrbms_remap_blocks', 'lrbms_peer_push',
 ]
 
 VEC_ONE, VEC_UI, VEC_UN, VEC_UR = 0, 1, 2, 3
@@ -128,6 +129,9 @@ def load_library():
             'lrbms_peer_push': (C.c_int, [vp, vp, i64, i32, vp, i32, vp]),
             'lrbms_pcg_workspace_bytes': (C.c_int, [vp, i64, P(C.c_size_t)]),
             'lrbms_pcg_solve': (C.c_int, [vp, i32, vp, vp, vp, vp, vp, dbl, i32, P(i32), P(dbl), vp, C.c_size_t, vp]),
+            'lrbms_affine_pcg_workspace_bytes': (C.c_int, [vp, i64, i64, P(C.c_size_t)]),
+            'lrbms_affine_pcg_solve': (C.c_int, [vp, i32, i32, vp, vp, vp, i32, vp, i64, vp, vp, i32, dbl, i32, i32,
+                                                 vp, vp, vp, vp, C.c_size_t, vp]),
         }
         for name, (res, args) in protos.items():
             fn = getattr(lib, name)          # AttributeError here = header/library mismatch

@@ -52,9 +52,94 @@ class BlockSwipdgDiscretization:
     def parse_parameter(self, mu):
         return parse_parameter(mu, self.parameter_type)
 
-    def solve(self, mu=None):
-        raise NotImplementedError('the fine-scale (FOM) solve runs in dune-gdt / ISTL in the reference and is outside '
-                                  'the LRBMS hot path (SURVEY.md section 2.1 #3); solve the reduced model instead')
+    #: device workspace bytes one call of the batched fine-scale solve may use; larger batches are solved in chunks
+    #: (each parameter's result does not depend on the chunking)
+    fom_workspace_budget = 4 << 30
+
+    def affine_system(self, subdomains):
+        """The affine components of the operator restricted to ``subdomains`` (in that order) on ONE sparsity pattern:
+        ``(pattern, values, rhs)`` with ``pattern`` a :class:`DeviceCsr` (its ``values`` are scratch for the caller),
+        ``values`` the ``(Q, nnz)`` component values and ``rhs`` the ``(Qf, n)`` right-hand side terms, all in HBM, so
+        that ``A(mu) = sum_q theta_q A_q`` is one pass over Q value arrays on the device.  Built once per subdomain tuple;
+        the union pattern is formed on the device from (row * n + column) keys."""
+        import scipy.sparse as sp
+        import torch
+        key = tuple(int(k) for k in subdomains)
+        cache = self.__dict__.setdefault('_affine_cache', {})
+        if key not in cache:
+            keys, datas, n_nb = [], [], 0
+            for op in self.operator.operators:
+                blocks = [[(op._blocks[k, l].csr.host if op._blocks[k, l] is not None else None) for l in key] for k in key]
+                M = sp.bmat(blocks, format='csr')
+                M.sum_duplicates()
+                n_nb = M.shape[0]
+                kk = np.repeat(np.arange(n_nb, dtype=np.int64), np.diff(M.indptr)) * n_nb + M.indices
+                keys.append(torch.from_numpy(kk).cuda())
+                datas.append(torch.from_numpy(np.ascontiguousarray(M.data, dtype=np.float64)).cuda())
+            key_p = torch.unique(torch.cat(keys), sorted=True)
+            vals = torch.zeros((len(keys), key_p.numel()), dtype=torch.float64, device='cuda')
+            for q in range(len(keys)):
+                vals[q, torch.searchsorted(key_p, keys[q])] = datas[q]
+            rows_p = torch.div(key_p, n_nb, rounding_mode='floor')
+            rowptr = torch.zeros(n_nb + 1, dtype=torch.int64, device='cuda')
+            rowptr[1:] = torch.cumsum(torch.bincount(rows_p, minlength=n_nb), 0)
+            A_dev = DeviceCsr.from_device(rowptr.to(torch.int32), (key_p - rows_p * n_nb).to(torch.int32), vals[0].clone(),
+                                          (n_nb, n_nb))
+            f = torch.stack([torch.cat([torch.from_numpy(o._array._blocks[k].to_numpy()[0]).cuda() for k in key])
+                             for o in self.rhs.operators]).contiguous()
+            cache[key] = (A_dev, vals, f)
+        return cache[key]
+
+    def solve(self, mu=None, inverse_options=None):
+        """``d.solve(mu)``: the fine-scale solution for one parameter (reference ``LincombOperator.assemble(mu)`` +
+        ``apply_inverse``, dune-istl); a block array of length 1.  See :meth:`solve_batch`."""
+        return self.solve_batch(None if mu is None and not self.parameter_type else [self.parse_parameter(mu)],
+                                inverse_options=inverse_options)
+
+    def solve_batch(self, mus, inverse_options=None):
+        """Fine-scale solutions for a parameter batch with the mu-batched Jacobi-preconditioned CG
+        (``lrbms_affine_pcg_solve``), from a zero initial guess.  ``inverse_options`` may hold ``rtol`` (true relative
+        residual, default 1e-9: the FP64 rounding of b - A x alone leaves up to ~1e-10 at C2, n = 393 216),
+        ``maxiter`` (default max(100, 10 n)) and ``restarts`` (default 3).  Returns a :class:`BlockVectorArray` of length
+        ``len(mus)`` whose blocks are views of one dof-major result buffer.
+        ``self.last_solve_info`` holds the per-parameter ``iterations``, ``relative_residual`` and ``status``
+        (0 converged, 1 not converged, 2 operator not positive definite); any non-zero status raises
+        :class:`LrbmsError` and no solution is returned."""
+        import torch
+        from ._lib import LrbmsError
+        from .kernels import affine_pcg_solve, affine_pcg_workspace_bytes
+        from .parameters import theta_matrix
+        from .vectorarray import BlockVectorArray, _round_cap
+        S = len(self.solution_space.subspaces)
+        pattern, values, rhs = self.affine_system(range(S))
+        coeffs = list(self.operator.coefficients) + list(self.rhs.coefficients)
+        theta = torch.from_numpy(theta_matrix(coeffs, mus, self.parameter_type)).cuda()
+        n, n_mu = pattern.shape[0], theta.shape[0]
+        opts = dict(inverse_options or {})
+        rtol = float(opts.get('rtol', 1e-9))
+        maxiter = int(opts['maxiter']) if opts.get('maxiter') is not None else max(100, 10 * n)
+        restarts = int(opts.get('restarts', 3))
+        buf = torch.zeros((n, _round_cap(n_mu)), dtype=torch.float64, device='cuda')
+        per_32 = affine_pcg_workspace_bytes(n, 32)
+        chunk = max(1, int(self.fom_workspace_budget * 32 // per_32))
+        info = {k: np.zeros(n_mu, dtype=dt) for k, dt in (('iterations', np.int32), ('relative_residual', np.float64),
+                                                            ('status', np.int32))}
+        for c0 in range(0, n_mu, chunk):
+            c1 = min(n_mu, c0 + chunk)
+            _, it, rr, st = affine_pcg_solve(pattern, values, rhs, theta[c0:c1], buf[:, c0:], rtol, maxiter, restarts)
+            info['iterations'][c0:c1], info['relative_residual'][c0:c1], info['status'][c0:c1] = it, rr, st
+        self.last_solve_info = info
+        bad = np.flatnonzero(info['status'])
+        if bad.size:
+            k = int(bad[0])
+            raise LrbmsError('fine-scale solve failed for parameter #{}: status {} ({}), relative residual {:.3e} '
+                             '(rtol {:.1e}) after {} iterations'.format(
+                                 k, int(info['status'][k]), {1: 'not converged', 2: 'operator not positive definite'}
+                                 .get(int(info['status'][k]), 'unknown'), info['relative_residual'][k], rtol,
+                                 int(info['iterations'][k])))
+        offs = np.concatenate([[0], np.cumsum([s.dim for s in self.solution_space.subspaces])])
+        blocks = [sub.from_dofmajor(buf[offs[i]:offs[i + 1]], n_mu) for i, sub in enumerate(self.solution_space.subspaces)]
+        return BlockVectorArray(blocks, self.solution_space)
 
     def estimate(self, U, mu=None, decompose=False):
         """Estimate for a *fine-scale* block array ``U`` through the generic operator chain, one parameter at a time,
@@ -71,37 +156,11 @@ class BlockSwipdgDiscretization:
         one-sided coupling terms the diagonal blocks carry on the outer interfaces act as the weakly imposed homogeneous
         Dirichlet condition of the oversampling problem.  The solve runs on the GPU (``lrbms_pcg_solve``);
         ``inverse_options`` may hold ``{'rtol': ..., 'maxiter': ...}``.  ``Us`` is accepted for signature parity."""
-        import scipy.sparse as sp
-        import torch
-        from .kernels import DeviceCsr, pcg_solve
+        from .kernels import pcg_solve
         mu = self.parse_parameter(mu)
         nb = list(self.neighborhoods[subdomain])
-        cache = self.__dict__.setdefault('_nbh_cache', {})
-        if subdomain not in cache:
-            # once per neighbourhood: the components A_q^nbh on ONE common sparsity pattern, values resident in HBM, so that
-            # A(mu) = sum_q theta_q A_q is one pass over Q value arrays on the device (no host sparse algebra per solve).
-            # The union pattern is formed on the device from (row * n + column) keys.
-            keys, datas, n_nb = [], [], 0
-            for op in self.operator.operators:
-                blocks = [[(op._blocks[k, l].csr.host if op._blocks[k, l] is not None else None) for l in nb] for k in nb]
-                M = sp.bmat(blocks, format='csr')
-                M.sum_duplicates()
-                n_nb = M.shape[0]
-                key = np.repeat(np.arange(n_nb, dtype=np.int64), np.diff(M.indptr)) * n_nb + M.indices
-                keys.append(torch.from_numpy(key).cuda())
-                datas.append(torch.from_numpy(np.ascontiguousarray(M.data, dtype=np.float64)).cuda())
-            key_p = torch.unique(torch.cat(keys), sorted=True)
-            vals = torch.zeros((len(keys), key_p.numel()), dtype=torch.float64, device='cuda')
-            for q in range(len(keys)):
-                vals[q, torch.searchsorted(key_p, keys[q])] = datas[q]
-            rows_p = torch.div(key_p, n_nb, rounding_mode='floor')
-            rowptr = torch.zeros(n_nb + 1, dtype=torch.int64, device='cuda')
-            rowptr[1:] = torch.cumsum(torch.bincount(rows_p, minlength=n_nb), 0)
-            A_dev = DeviceCsr.from_device(rowptr.to(torch.int32), (key_p - rows_p * n_nb).to(torch.int32), vals[0].clone(),
-                                          (n_nb, n_nb))
-            f = torch.cat([torch.from_numpy(self.rhs.operators[0]._array._blocks[k].to_numpy()[0]).cuda() for k in nb])
-            cache[subdomain] = (A_dev, vals, f)
-        A_dev, vals_q, f = cache[subdomain]
+        A_dev, vals_q, f = self.affine_system(nb)
+        f = f[0]
         theta = [c.evaluate(mu) if hasattr(c, 'evaluate') else float(c) for c in self.operator.coefficients]
         values = float(theta[0]) * vals_q[0]
         for q in range(1, vals_q.shape[0]):

@@ -149,3 +149,38 @@ def pcg_solve(csr, b, x0=None, rtol=1e-12, max_iter=None):
                                   int(max_iter if max_iter is not None else max(100, 10 * n)), C.byref(iters), C.byref(relres),
                                   ws.data_ptr(), nbytes.value, current_stream_ptr()))
     return x, iters.value, relres.value
+
+
+def affine_pcg_workspace_bytes(n, n_mu):
+    """Device workspace ``lrbms_affine_pcg_solve`` needs for ``n_mu`` parameters of an ``n``-dof system."""
+    import ctypes as C
+    h = Handle.get()
+    nbytes = C.c_size_t()
+    h.check(h.lib.lrbms_affine_pcg_workspace_bytes(h.h, int(n), int(n_mu), C.byref(nbytes)))
+    return nbytes.value
+
+
+def affine_pcg_solve(pattern, values, rhs, theta, x, rtol, max_iter, max_restarts):
+    """Solve ``(sum_q theta[k, q] A_q) x_k = sum_f theta[k, Q + f] rhs_f`` for every row ``k`` of ``theta`` with
+    ``lrbms_affine_pcg_solve``.  ``pattern``: :class:`DeviceCsr` whose ``rowptr`` / ``colind`` every component shares;
+    ``values``: ``(Q, nnz)`` and ``rhs``: ``(Qf, n)`` float64 CUDA tensors; ``theta``: ``(n_mu, Q + Qf)`` CUDA tensor;
+    ``x``: dof-major ``(n, >= n_mu)`` CUDA view (row stride ``ld``), initial guess in, solution out.
+    Returns ``(x, iterations, true relative residual, status)``, the last three host arrays of length ``n_mu``."""
+    import ctypes as C
+    from ._lib import current_stream_ptr, ptr
+    torch = _torch()
+    n, n_mu = pattern.shape[0], theta.shape[0]
+    Q, Qf = values.shape[0], rhs.shape[0]
+    assert values.is_contiguous() and rhs.is_contiguous() and theta.is_contiguous() and theta.shape[1] == Q + Qf
+    assert x.shape[0] == n and x.shape[1] >= n_mu and x.stride(1) == 1
+    h = Handle.get()
+    nbytes = affine_pcg_workspace_bytes(n, n_mu)
+    ws = torch.empty(max(1, nbytes // 8), dtype=torch.float64, device='cuda')
+    iters = np.zeros(n_mu, dtype=np.int32)
+    relres = np.zeros(n_mu, dtype=np.float64)
+    status = np.zeros(n_mu, dtype=np.int32)
+    h.check(h.lib.lrbms_affine_pcg_solve(h.h, n, Q, ptr(pattern.rowptr), ptr(pattern.colind), ptr(values), Qf, ptr(rhs),
+                                         n_mu, ptr(theta), ptr(x), x.stride(0), float(rtol), int(max_iter),
+                                         int(max_restarts), ptr(iters), ptr(relres), ptr(status), ptr(ws), nbytes,
+                                         current_stream_ptr()))
+    return x, iters, relres, status

@@ -61,6 +61,17 @@ def parse_parameter_batch(mus, parameter_type):
     return out, arr.shape[0]
 
 
+def theta_matrix(coefficients, mus, parameter_type):
+    """``(n_mu, len(coefficients))`` matrix of the coefficients evaluated on a parameter batch (``mus=None``: one row
+    for a parameter-independent model) -- the layout the mu-batched kernels read."""
+    if mus is None:
+        return np.array([[float(c) if not isinstance(c, ParameterFunctional) else c.evaluate(None) for c in coefficients]])
+    batch, n_mu = parse_parameter_batch(mus, parameter_type)
+    cols = [c.evaluate_batch(batch, n_mu) if isinstance(c, ParameterFunctional) else np.full(n_mu, float(c))
+            for c in coefficients]
+    return np.ascontiguousarray(np.stack(cols, axis=1))
+
+
 class ParameterFunctional:
     def evaluate(self, mu=None):
         raise NotImplementedError

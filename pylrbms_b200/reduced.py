@@ -21,7 +21,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import Handle, LrbmsError, current_stream_ptr, host_f64, host_i32, ptr
-from .parameters import ParameterFunctional, ProductParameterFunctional, parse_parameter, parse_parameter_batch
+from .parameters import ParameterFunctional, ProductParameterFunctional, parse_parameter, theta_matrix
 from .vectorarray import ReducedVectorArray
 
 
@@ -244,12 +244,7 @@ class ReducedModel:
     # -- coefficient evaluation on the host (theta_q are tiny expressions; reference: ExpressionParameterFunctional)
     def thetas(self, mus):
         """``(n_mu, Q + Qf)`` coefficient matrix for a parameter batch."""
-        coeffs = list(self.operator.coefficients) + list(self.rhs.coefficients)
-        if mus is None:
-            return np.array([[float(c) if not isinstance(c, ParameterFunctional) else c.evaluate(None) for c in coeffs]])
-        batch, n_mu = parse_parameter_batch(mus, self.parameter_type)
-        cols = [c.evaluate_batch(batch, n_mu) if isinstance(c, ParameterFunctional) else np.full(n_mu, float(c)) for c in coeffs]
-        return np.ascontiguousarray(np.stack(cols, axis=1))
+        return theta_matrix(list(self.operator.coefficients) + list(self.rhs.coefficients), mus, self.parameter_type)
 
     # -- online plan -------------------------------------------------------------------------------------
     def _theta_index(self, functional, lam):
