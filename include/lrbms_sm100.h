@@ -320,6 +320,53 @@ int lrbms_affine_pcg_solve(lrbms_handle_t h, int32_t n, int32_t Q, const int32_t
                            int32_t* iters_out, double* relres_out, int32_t* status_out,
                            void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------------------------- */
+/*  Reduction error of a parameter batch (reduction_error_analysis; the reference's "max discretization    */
+/*  error" loop, scripts/online_adaptive_lrbms.py:49-53,141-143: reductor.reconstruct(rd.solve(mu)), the   */
+/*  difference to d.solve(mu) and its norm, one mu and one subdomain at a time).                          */
+/* ---------------------------------------------------------------------------------------------------- */
+/* One subdomain of the reconstruction: rows row_offset .. row_offset + n_rows of u_h / e, the local basis V (device,
+ * dof-major n_rows x ldv, len vectors) and the first N of its vectors (N = block_dims[i] of the reduced solution, which may
+ * be smaller than len for a solution of an older reduced model; N > len is LRBMS_ERR_INVALID), whose coefficients sit in
+ * columns red_offset .. red_offset + N of u_N.  Blocks are in ascending, disjoint row order. */
+typedef struct {
+  const double* V;
+  int32_t ldv;
+  int32_t len;
+  int32_t N;
+  int32_t red_offset;
+  int64_t row_offset;
+  int32_t n_rows;
+  int32_t reserved;
+} lrbms_recon_block_t;
+/* e[r][m] = u_h[r][m] - sum_{k < N_i} V_i[r - row_offset_i][k] * u_N[m][red_offset_i + k], k ascending, for every row of
+ * every block and every m < n_mu, in one launch.  u_h: device, dof-major rows x ldu (the buffer of d.solve_batch, column =
+ * parameter; columns n_mu .. ldu are not read); u_N: device, row-major n_mu x ldn, n_red used columns (the reduced
+ * solutions); e: device, dof-major rows x lde, written for m < n_mu only (it may not alias u_h).  ldu, lde < n_mu or
+ * ldn < n_red are LRBMS_ERR_INVALID.  A block with N = 0 gets e = u_h.  Every entry is one sequential fma chain: a
+ * parameter's bits do not depend on the batch.  lrbms_recon_error_workspace_bytes: device workspace for n_mu parameters of
+ * n_red reduced coefficients (a transposed copy of u_N, the block table and the row partition). */
+int lrbms_recon_error_workspace_bytes(lrbms_handle_t h, int32_t n_sub, const lrbms_recon_block_t* blocks_host, int64_t n_mu,
+                                      int32_t n_red, size_t* bytes);
+int lrbms_recon_error(lrbms_handle_t h, int32_t n_sub, const lrbms_recon_block_t* blocks_host, int64_t n_mu,
+                      const double* u_h, int32_t ldu, const double* u_N, int32_t n_red, int32_t ldn, double* e, int32_t lde,
+                      void* workspace, size_t workspace_bytes, void* stream);
+/* Segmented affine quadratic form: out[s][m] = sum_{seg_ptr[s] <= r < seg_ptr[s+1]} x[r][m] sum_c (sum_q theta[m][q]
+ * A_q[r][c]) x[c][m] for the n_seg row segments (host seg_ptr [n_seg + 1], non-decreasing within [0, n]).  The Q
+ * components share ONE CSR pattern (rowptr [n + 1], colind [nnz], values [Q][nnz]; 1 <= Q <= 4, else
+ * LRBMS_ERR_UNSUPPORTED); theta: device, row-major n_mu x ldt, the first Q columns read (ldt < Q is LRBMS_ERR_INVALID), or
+ * NULL for theta = 1 with Q = 1 (a plain product matrix).  x: device, dof-major n x ldx (ldx >= n_mu); out: device, n_seg x
+ * ldo (ldo >= n_mu).  Used with the block-diagonal local energy products (segments = subdomains: local squared norms) and
+ * with the affine system operator (one segment: |||x|||_mu^2; per-subdomain row partials of a coupled operator are not
+ * norms).  Row sums run in CSR order inside one lane, rows are added per warp, warp and CTA in a fixed order over a row
+ * partition set by the segment sizes and the SM count only: a parameter's bits do not depend on the batch.  No atomics.
+ * lrbms_segmented_form_workspace_bytes: device workspace (CTA partials of 256 parameters and the partition). */
+int lrbms_segmented_form_workspace_bytes(lrbms_handle_t h, int32_t n_seg, const int32_t* seg_ptr_host, size_t* bytes);
+int lrbms_segmented_form(lrbms_handle_t h, int32_t n, int32_t Q, const int32_t* rowptr, const int32_t* colind,
+                         const double* values, int64_t nnz, int32_t n_seg, const int32_t* seg_ptr_host, int64_t n_mu,
+                         const double* theta, int32_t ldt, const double* x, int32_t ldx, double* out, int32_t ldo,
+                         void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

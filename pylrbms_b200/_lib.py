@@ -24,6 +24,7 @@ EXPORTS = [
     'lrbms_online_plan_create', 'lrbms_online_workspace_bytes', 'lrbms_online_solve', 'lrbms_online_estimate',
     'lrbms_online_sweep', 'lrbms_eta_max', 'lrbms_online_debug_timing',
     'lrbms_pcg_workspace_bytes', 'lrbms_pcg_solve', 'lrbms_affine_pcg_workspace_bytes', 'lrbms_affine_pcg_solve',
+    'lrbms_recon_error_workspace_bytes', 'lrbms_recon_error', 'lrbms_segmented_form_workspace_bytes', 'lrbms_segmented_form',
     'lrbms_remap_blocks', 'lrbms_peer_push',
 ]
 
@@ -57,6 +58,11 @@ class RemapDesc(C.Structure):
     _fields_ = [('dst', C.c_void_p), ('NL', C.c_int32), ('NR', C.c_int32), ('prev', C.c_void_p), ('pNR', C.c_int32),
                 ('n_cn', C.c_int32), ('cols_new', C.c_void_p), ('rows_new', C.c_void_p), ('n_rn', C.c_int32),
                 ('reserved', C.c_int32), ('row_map', C.c_void_p), ('col_map', C.c_void_p)]
+
+
+class ReconBlock(C.Structure):
+    _fields_ = [('V', C.c_void_p), ('ldv', C.c_int32), ('len', C.c_int32), ('N', C.c_int32), ('red_offset', C.c_int32),
+                ('row_offset', C.c_int64), ('n_rows', C.c_int32), ('reserved', C.c_int32)]
 
 
 class EstimatorTerm(C.Structure):
@@ -132,6 +138,11 @@ def load_library():
             'lrbms_affine_pcg_workspace_bytes': (C.c_int, [vp, i64, i64, P(C.c_size_t)]),
             'lrbms_affine_pcg_solve': (C.c_int, [vp, i32, i32, vp, vp, vp, i32, vp, i64, vp, vp, i32, dbl, i32, i32,
                                                  vp, vp, vp, vp, C.c_size_t, vp]),
+            'lrbms_recon_error_workspace_bytes': (C.c_int, [vp, i32, vp, i64, i32, P(C.c_size_t)]),
+            'lrbms_recon_error': (C.c_int, [vp, i32, vp, i64, vp, i32, vp, i32, i32, vp, i32, vp, C.c_size_t, vp]),
+            'lrbms_segmented_form_workspace_bytes': (C.c_int, [vp, i32, vp, P(C.c_size_t)]),
+            'lrbms_segmented_form': (C.c_int, [vp, i32, i32, vp, vp, vp, i64, i32, vp, i64, vp, i32, vp, i32, vp, i32,
+                                               vp, C.c_size_t, vp]),
         }
         for name, (res, args) in protos.items():
             fn = getattr(lib, name)          # AttributeError here = header/library mismatch

@@ -184,3 +184,58 @@ def affine_pcg_solve(pattern, values, rhs, theta, x, rtol, max_iter, max_restart
                                          int(max_restarts), ptr(iters), ptr(relres), ptr(status), ptr(ws), nbytes,
                                          current_stream_ptr()))
     return x, iters, relres, status
+
+
+def recon_error(bases, block_dims, u_h, u_N, e):
+    """``e = u_h - R u_N`` for all subdomains in one launch (``lrbms_recon_error``).  ``bases``: the local bases (one
+    :class:`GpuVectorArray` per subdomain, in row order); ``block_dims``: the coefficients per subdomain in ``u_N`` (the first
+    ``block_dims[i]`` vectors of basis ``i`` are used); ``u_h`` / ``e``: dof-major ``(n, >= n_mu)`` CUDA views; ``u_N``:
+    ``(n_mu, n_red)`` CUDA tensor with unit column stride.  Returns ``e``."""
+    import ctypes as C
+    from ._lib import ReconBlock, current_stream_ptr, ptr
+    torch = _torch()
+    n_mu, n_red = u_N.shape
+    assert len(bases) == len(block_dims) and u_N.stride(1) == 1 and u_h.stride(1) == 1 and e.stride(1) == 1
+    assert u_h.shape[0] == e.shape[0] and u_h.shape[1] >= n_mu and e.shape[1] >= n_mu
+    blocks = (ReconBlock * max(1, len(bases)))()
+    row, red = 0, 0
+    for i, (V, N) in enumerate(zip(bases, block_dims)):
+        blocks[i] = ReconBlock(V.device_ptr, V.ld, len(V), int(N), red, row, V.dim, 0)
+        row, red = row + V.dim, red + int(N)
+    assert row == u_h.shape[0], 'the bases do not cover the rows of u_h'
+    h = Handle.get()
+    nbytes = C.c_size_t()
+    h.check(h.lib.lrbms_recon_error_workspace_bytes(h.h, len(bases), C.cast(blocks, C.c_void_p), n_mu, n_red, C.byref(nbytes)))
+    ws = torch.empty(max(1, nbytes.value // 8 + 1), dtype=torch.float64, device='cuda')
+    h.check(h.lib.lrbms_recon_error(h.h, len(bases), C.cast(blocks, C.c_void_p), n_mu, ptr(u_h), u_h.stride(0), ptr(u_N),
+                                    n_red, max(n_red, u_N.stride(0)), ptr(e), e.stride(0), ptr(ws),
+                                    ws.numel() * 8, current_stream_ptr()))
+    return e
+
+
+def segmented_form(pattern, values, seg_ptr, x, n_mu, theta=None, out=None):
+    """``out[s, m] = sum over the rows of segment s of x[r, m] (sum_q theta[m, q] A_q x[:, m])[r]``
+    (``lrbms_segmented_form``).  ``pattern``: :class:`DeviceCsr` whose ``rowptr`` / ``colind`` the components share;
+    ``values``: ``(Q, nnz)`` CUDA tensor; ``seg_ptr``: host row offsets of the segments; ``x``: dof-major ``(n, >= n_mu)``
+    CUDA view; ``theta``: ``(n_mu, >= Q)`` CUDA tensor with unit column stride, or None for theta = 1 (Q = 1).
+    Returns ``out``, an ``(n_seg, n_mu)`` CUDA tensor."""
+    import ctypes as C
+    from ._lib import current_stream_ptr, host_i32, ptr
+    torch = _torch()
+    seg = host_i32(seg_ptr)
+    n_seg = seg.size - 1
+    Q, nnz = values.shape
+    assert values.is_contiguous() and x.stride(1) == 1 and x.shape[0] == pattern.shape[0]
+    if theta is not None:
+        assert theta.shape[0] >= n_mu and theta.stride(1) == 1
+    if out is None:
+        out = torch.empty((n_seg, max(1, n_mu)), dtype=torch.float64, device='cuda')[:, :n_mu]
+    h = Handle.get()
+    nbytes = C.c_size_t()
+    h.check(h.lib.lrbms_segmented_form_workspace_bytes(h.h, n_seg, ptr(seg), C.byref(nbytes)))
+    ws = torch.empty(max(1, nbytes.value // 8 + 1), dtype=torch.float64, device='cuda')
+    h.check(h.lib.lrbms_segmented_form(h.h, pattern.shape[0], Q, ptr(pattern.rowptr), ptr(pattern.colind), ptr(values), nnz,
+                                       n_seg, ptr(seg), int(n_mu), ptr(theta),
+                                       theta.stride(0) if theta is not None else 0, ptr(x), x.stride(0), ptr(out),
+                                       out.stride(0), ptr(ws), ws.numel() * 8, current_stream_ptr()))
+    return out
