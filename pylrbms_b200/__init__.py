@@ -20,3 +20,4 @@ from .reduced import ReducedModel, ReducedBlockOperator                         
 __version__ = '0.1.0'
 from .online_enrichment import AdaptiveEnrichment, doerfler_marking                              # noqa: F401
 from .error_analysis import reduction_error_analysis, ReductionErrorAnalysis                     # noqa: F401
+from .greedy import greedy                                                                       # noqa: F401

@@ -101,7 +101,19 @@ class GenericRBSystemReductor:
             return float(v.pairwise_dot(v)[0])
         return float(product.pairwise_apply2(v, v)[0])
 
-    def extend_basis(self, U):
+    def extend_basis(self, U, method='gram_schmidt', pod_modes=1, pod_rtol=1e-13):
+        """Extend every local basis by the restrictions of the block array ``U`` (pyMOR ``extend_basis``).
+
+        ``method='gram_schmidt'``: each restriction goes through :meth:`extend_basis_local`, vector by vector.
+        ``method='pod'``: all subdomains at once -- the projection error of ``U`` onto the current bases (two classical
+        Gram-Schmidt passes in the local product), a POD of it per subdomain and at most ``pod_modes`` modes appended
+        whose singular value exceeds ``pod_rtol`` times the largest local norm of ``U``; the modes are orthonormalised
+        against the basis and among themselves (pyMOR ``pod_orthonormalize=True``).  See :func:`_extend_basis_pod`.
+        Either way :class:`ExtensionError` is raised when no subdomain received a vector."""
+        if method == 'pod':
+            return _extend_basis_pod(self, U, int(pod_modes), float(pod_rtol))
+        if method != 'gram_schmidt':
+            raise ValueError("extend_basis: method must be 'gram_schmidt' or 'pod', not {!r}".format(method))
         ok = False
         for blk in U._blocks:
             try:
@@ -137,6 +149,160 @@ class GenericRBSystemReductor:
 
     def reduce(self):
         return self._reduce()
+
+
+# ----------------------------------------------------------------------------------------------------------
+#  POD extension of every local basis in one pass
+# ----------------------------------------------------------------------------------------------------------
+
+def _run_project(descs, keep):
+    """One projection plan over ``descs`` (at most one descriptor per subdomain and quantity), run once."""
+    if descs:
+        plan = make_project_plan(Handle.get(), descs, keep)
+        plan.run()
+        plan.destroy()
+
+
+def _inner_with_bases(csrs, Xs, bases, width):
+    """``C[m, off_i + j] = <x_{i,m}, v_{i,j}>_{P_i}`` for all subdomains with one projection plan: ``(width, sum N_i)``, the
+    coefficient layout of ``lrbms_recon_error``."""
+    torch = _torch()
+    offs = np.concatenate([[0], np.cumsum([len(V) for V in bases])]).astype(np.int64)
+    C = torch.zeros((width, int(offs[-1])), dtype=torch.float64, device='cuda')
+    descs = [project_desc(csr, X.dim, X.device_ptr, X.ld, len(X), V.device_ptr, V.ld, len(V), C.data_ptr() + 8 * int(offs[i]),
+                          int(offs[-1])) for i, (csr, X, V) in enumerate(zip(csrs, Xs, bases)) if len(X) and len(V)]
+    _run_project(descs, [C])
+    return C
+
+
+def _grams(csrs, arrays_list, width):
+    """``G[t, i] = X_i^T P_i X_i`` (``width x width``, leading ``len(X_i)`` rows / columns) for every array list ``t`` and
+    subdomain ``i``, symmetric descriptors, one projection plan; returned on the host."""
+    torch = _torch()
+    S = len(csrs)
+    G = torch.zeros((len(arrays_list), S, width, width), dtype=torch.float64, device='cuda')
+    descs = []
+    for t, Xs in enumerate(arrays_list):
+        for i, (csr, X) in enumerate(zip(csrs, Xs)):
+            if len(X):
+                descs.append(project_desc(csr, X.dim, X.device_ptr, X.ld, len(X), X.device_ptr, X.ld, len(X),
+                                          G[t, i].data_ptr(), width, symmetric=csr is None or csr.symmetric))
+    _run_project(descs, [G])
+    G = G.cpu().numpy()
+    return 0.5 * (G + np.swapaxes(G, -1, -2))
+
+
+def _combine(views, counts, coeffs):
+    """``Y_i = X_i A_i`` for every subdomain in one ``lrbms_recon_error`` launch: ``views[i]`` holds ``counts[i]`` columns,
+    ``coeffs[i]`` is ``(counts[i], m_i)``.  Returns the dof-major ``(n, >= max m_i)`` result; columns past ``m_i`` of a
+    subdomain are zero."""
+    torch = _torch()
+    from .kernels import recon_error
+    from .vectorarray import _round_cap
+    width = max(a.shape[1] for a in coeffs)
+    offs = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    coef = np.zeros((width, int(offs[-1])))
+    for i, a in enumerate(coeffs):
+        coef[:a.shape[1], offs[i]:offs[i + 1]] = -a.T             # e = 0 - X (-A) = X A
+    n = sum(X.dim for X in views)
+    zero = torch.zeros((n, _round_cap(width)), dtype=torch.float64, device='cuda')
+    Y = torch.empty((n, _round_cap(width)), dtype=torch.float64, device='cuda')
+    return recon_error(views, counts, zero, torch.from_numpy(coef).cuda(), Y)
+
+
+def _views(subs, rows, X, counts):
+    """The subdomain blocks of a dof-major ``(n, >= max counts)`` buffer as arrays of ``counts[i]`` vectors (no copy)."""
+    return [s.from_dofmajor(X[rows[i]:rows[i + 1]], counts[i]) for i, s in enumerate(subs)]
+
+
+def _subtract_projection(subs, rows, csrs, bases, X, counts):
+    """``X_i - V_i (V_i^T P_i X_i)`` for every subdomain: one projection plan and one ``lrbms_recon_error`` launch."""
+    torch = _torch()
+    from .kernels import recon_error
+    from .vectorarray import _round_cap
+    width = max(counts)
+    C = _inner_with_bases(csrs, _views(subs, rows, X, counts), bases, width)
+    out = torch.zeros((X.shape[0], _round_cap(width)), dtype=torch.float64, device='cuda')
+    if C.shape[1] == 0:                      # every basis is empty
+        out[:, :width] = X[:, :width]
+        return out
+    return recon_error(bases, [len(V) for V in bases], X, C, out)
+
+
+def pod_modes_from_gram(G, norm_max, pod_modes, pod_rtol):
+    """Host half of the POD extension for one subdomain: ``(W, sigma)`` of the at most ``pod_modes`` leading eigenpairs of
+    the Gram matrix ``G`` of the projection error with ``sigma > pod_rtol * norm_max``, in descending order, each
+    eigenvector signed so that its entry of largest magnitude is positive."""
+    lam, W = np.linalg.eigh(G)
+    lam, W = lam[::-1], W[:, ::-1]
+    sigma = np.sqrt(np.maximum(lam, 0.0))
+    m = min(int(pod_modes), int(np.count_nonzero(sigma > pod_rtol * norm_max)))
+    W, sigma = W[:, :m].copy(), sigma[:m]
+    for j in range(m):
+        if W[np.argmax(np.abs(W[:, j])), j] < 0:
+            W[:, j] = -W[:, j]
+    return W, sigma
+
+
+def cholesky_leading(G):
+    """Lower Cholesky factor of the largest leading block of ``G`` that is numerically positive definite: ``(m, L)``.
+    A mode that the re-orthogonalisation reduced to rounding noise is dropped with everything after it."""
+    for m in range(G.shape[0], 0, -1):
+        try:
+            return m, np.linalg.cholesky(G[:m, :m])
+        except np.linalg.LinAlgError:
+            continue
+    return 0, np.zeros((0, 0))
+
+
+def _extend_basis_pod(reductor, U, pod_modes, pod_rtol):
+    """``extend_basis(U, method='pod')`` on the device.  Per subdomain ``i`` (``U_i``: restriction of ``U``, ``V_i``: basis,
+    ``P_i``: the reductor's product, the Euclidean one when it is None):
+
+    1. ``R = U - V (V^T P U)`` twice (CGS2): one projection plan and one ``lrbms_recon_error`` launch per pass;
+    2. ``G_i = R_i^T P_i R_i`` and ``U_i^T P_i U_i`` in one plan, to the host;
+    3. host ``eigh``: at most ``pod_modes`` modes with ``sigma > pod_rtol max_j |u_{i,j}|_{P_i}``;
+    4. ``Y_i = R_i W_i / sigma_i`` (one launch), one more CGS pass against ``V``, Cholesky QR of ``Y_i^T P_i Y_i`` (one plan, one
+       launch), and the result is appended.
+
+    Returns the number of vectors appended to each basis; raises :class:`ExtensionError` when that is zero everywhere."""
+    from .error_analysis import _dofmajor
+    if pod_modes < 1:
+        raise ValueError('pod_modes must be at least 1')
+    subs = reductor.d.solution_space.subspaces
+    S, k = len(subs), len(U)
+    if len(U._blocks) != S or any(b.dim != s.dim for b, s in zip(U._blocks, subs)):
+        raise ValueError('U is not an array of the solution space of the reductor')
+    if k == 0:
+        raise ExtensionError
+    rows = np.concatenate([[0], np.cumsum([s.dim for s in subs])]).astype(np.int64)
+    n = int(rows[-1])
+    bases = [reductor.bases[s.id] for s in subs]
+    csrs = [p.csr if p is not None else None for p in reductor.products]
+    u = _dofmajor(U, n, k)
+    R = u
+    for _ in range(2):
+        R = _subtract_projection(subs, rows, csrs, bases, R, [k] * S)
+    views = lambda X, counts: _views(subs, rows, X, counts)
+    G, H = _grams(csrs, [views(R, [k] * S), views(u, [k] * S)], k)
+    modes = [pod_modes_from_gram(G[i], np.sqrt(np.maximum(np.diag(H[i]), 0.0)).max(), pod_modes, pod_rtol)
+             for i in range(S)]
+    counts = [W.shape[1] for W, _ in modes]
+    if max(counts) == 0:
+        raise ExtensionError
+    Y = _combine(views(R, [k] * S), [k] * S, [W / sigma for W, sigma in modes])
+    Y = _subtract_projection(subs, rows, csrs, bases, Y, counts)
+    Gy = _grams(csrs, [views(Y, counts)], max(counts))[0]
+    factors = [cholesky_leading(Gy[i, :counts[i], :counts[i]]) for i in range(S)]
+    counts = [m for m, _ in factors]
+    if max(counts) == 0:
+        raise ExtensionError
+    inv = [np.linalg.inv(L).T if m else np.zeros((0, 0)) for m, L in factors]   # Z = Y L^{-T}
+    Z = _combine(views(Y, counts), counts, inv)
+    for i, s in enumerate(subs):
+        if counts[i]:
+            bases[i].append(s.from_dofmajor(Z[rows[i]:rows[i + 1]], counts[i]))
+    return counts
 
 
 # ----------------------------------------------------------------------------------------------------------
